@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference algorithm on the host CPU (oracle port)
     torchrun ... bench.py --gpus N ...                       # one rank per GPU, frames sharded, no collective
+    python bench.py ... --dump-outputs DIR                   # + the frames of the last timed step as DIR/*.npy (see dump_outputs)
 
 Workload (`config.workload`; the same for both arms):
   N = 1   BASELINE config 2: a 32-frame GOF, 1024x1024 atlas, 10-bit geometry, 2 maps, occupancy precision 4, grid geometry
@@ -37,6 +38,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (which may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -71,6 +73,7 @@ class ClockSampler:
 
     def __init__(self, gpu_index: int):
         self.rows, self.proc, self.idx = [], None, gpu_index
+        self.paused = False
 
     def start(self):
         try:
@@ -84,7 +87,8 @@ class ClockSampler:
 
     def _read(self):
         for line in self.proc.stdout:
-            self.rows.append([c.strip() for c in line.split(",")])
+            if not self.paused:
+                self.rows.append([c.strip() for c in line.split(",")])
 
     def stop(self):
         if not self.proc:
@@ -220,6 +224,39 @@ def host_copy_ceiling(torch, dev, h2d_bytes, d2h_bytes, iters, barrier):
     return dt
 
 
+DUMP_POINTS = 1 << 20       # --dump-outputs: sampled points over all ranks (40 bytes each below, so DIR stays well under 64 MB)
+DUMP_SEED = 0x7C2D
+
+
+def dump_outputs(out_dir, frames, rank=0, world=1):
+    """Writes the frames a caller of the timed path receives, `frames` = [(positions u16 [n,3], colours u8 [n,3])], as .npy files:
+    every frame's point count and column sums over all of its points (float64), and a seeded sample of its points (float32)
+    with their (frame, point) indices.  A frame's sample depends on its place in `frames` and its point count only, so two
+    builds that agree on the counts sample the same points.  Under several ranks each rank writes rank<R>_*.npy and samples
+    its share of DUMP_POINTS."""
+    os.makedirs(out_dir, exist_ok=True)
+    prefix = f"rank{rank}_" if world > 1 else ""
+    per_frame = max(1, DUMP_POINTS // max(1, world) // max(1, len(frames)))
+    counts, sums, index, pos, col = [], [], [], [], []
+    for j, (p, c) in enumerate(frames):
+        n = len(p)
+        pick = np.arange(n)
+        if n > per_frame:
+            pick = np.sort(np.random.default_rng([DUMP_SEED, j]).choice(n, per_frame, replace=False))
+        counts.append(n)
+        sums.append(np.concatenate([p.sum(0, dtype=np.float64), c.sum(0, dtype=np.float64)]))
+        index.append(np.stack([np.full(len(pick), j), pick], 1))
+        pos.append(p[pick])
+        col.append(c[pick])
+    out = {"points_per_frame": np.array(counts, np.float64), "frame_sums": np.array(sums, np.float64).reshape(-1, 6),
+           "sample_index": np.concatenate(index).astype(np.float64).reshape(-1, 2),
+           "sample_positions": np.concatenate(pos).astype(np.float32).reshape(-1, 3),
+           "sample_colors": np.concatenate(col).astype(np.float32).reshape(-1, 3)}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -237,7 +274,11 @@ def main():
                     help="streams the kernel-only loop spreads its GOFs over (consecutive GOFs of a stream overlap: the small "
                          "latency-bound passes of one run under the emit of the other)")
     ap.add_argument("--quick", action="store_true", help="skip the secondary measurements (pageable e2e, one-context, host ceiling)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frames the last timed kernel-only step computed to DIR/*.npy "
+                                                          "(under several ranks: DIR/rank<R>_*.npy)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the CUDA path (--impl b200)")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -364,6 +405,12 @@ def main():
     e1.record(tstream)
     barrier()
     kernel_ms = e0.elapsed_time(e1) / inner               # per pass over the rank's GOF list
+    if args.dump_outputs:
+        # every resident of the plan was last launched in the last timed step: read them before anything relaunches one
+        last = list(dict.fromkeys(r for r, _ in plan))
+        sampler.paused = True                              # the clocks block covers the timed regions only
+        dump_outputs(args.dump_outputs, [r.fetch(f, int(n)) for r in last for f, n in enumerate(r.counts())], rank, world)
+        sampler.paused = False
     # per-stage device times (library-recorded CUDA events on the same stream), measured on separate launches so that
     # reading them does not serialise the timed loop above
     unpack_ms, stage_acc = [], {}
