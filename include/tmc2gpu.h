@@ -152,10 +152,28 @@ typedef struct tmc2_gof {
   uint32_t          frame_count;           /* frames to reconstruct (decoder.rs:188)                       */
   uint32_t          geo_video_frames;      /* atlas.geo_frames[0].frame_count(); must be >= 2*frame_count   */
   uint32_t          attr_video_frames;     /* atlas.attr_frames[0].frame_count()                           */
-  uint32_t          _reserved;
+  uint32_t          input_flags;           /* TMC2_INPUT_* bits; 0 = every plane in host memory            */
   const tmc2_frame* frames;                /* frame_count entries                                          */
   tmc2_params       params;
 } tmc2_gof;
+
+/* Where the planes of a GOF live and how they are laid out (tmc2_gof.input_flags).  Unknown bits -> TMC2_ERR_INVALID_ARG.
+ * TMC2_INPUT_DEVICE: every plane pointer of the GOF (occ, geo, attr_*) is CUDA device (or managed) memory on one of the
+ *   context's devices -- what NVDEC or ffmpeg's CUDA hwaccel hands out.  The planes are not copied through the host: one
+ *   kernel gathers them into the library's own layout.  Each plane is checked: host memory (tmc2gpu_alloc_pinned blocks
+ *   included) and a plane whose extent ((rows-1)*stride + row) runs past the end of its allocation -> TMC2_ERR_INVALID_ARG;
+ *   a plane on a device that the reconstructing device cannot reach by peer access -> TMC2_ERR_UNSUPPORTED.
+ * TMC2_INPUT_P010 (needs TMC2_INPUT_DEVICE, else TMC2_ERR_UNSUPPORTED): the 16-bit planes use the P010 layout that NVDEC
+ *   and ffmpeg's p010le write.  A sample's 10-bit value sits in bits 15..6 (the library reads raw >> 6, the low 6 bits are
+ *   ignored).  attr_u[m] is the interleaved UV plane, (width/2) x (height/2) pairs with U first, attr_stride_c counts u16
+ *   elements and must be >= width; attr_v[m] must be NULL.  geo[m] is the Y plane of the geometry frame (its chroma is
+ *   never read).  The occupancy plane stays plain u8 (the luma plane of an nv12 frame).
+ *
+ * Feeding AVFrames of ffmpeg's CUDA hwaccel (AV_PIX_FMT_CUDA, sw_format p010le for geometry / attributes, nv12 for
+ * occupancy): plane pointer = frame->data[0] (Y) / frame->data[1] (interleaved UV), stride in ELEMENTS = linesize[i] / 2
+ * for p010le and linesize[0] for the nv12 occupancy luma; set input_flags = TMC2_INPUT_DEVICE | TMC2_INPUT_P010.       */
+#define TMC2_INPUT_DEVICE 1u
+#define TMC2_INPUT_P010   2u
 
 /* ------------------------------------------------------------------------------------------------
  * One reconstructed frame == reference `PointSet3` (src/codec.rs:20-36): positions are
@@ -208,7 +226,10 @@ TMC2_API const char* tmc2gpu_status_string(tmc2_status s);
  * src/decoder.rs:1136-1140).  Planes inside a tmc2gpu_alloc_pinned block are read by the DMA engine IN PLACE after
  * submit_gof has returned: they must stay unmodified until tmc2gpu_wait_inputs returns (or until the first frame of that
  * GOF has been handed out by tmc2gpu_next_frame).  The patch lists and the tmc2_gof / tmc2_frame structs themselves are
- * only read during submit_gof.                                                                                      */
+ * only read during submit_gof.
+ * DEVICE PLANES (TMC2_INPUT_DEVICE).  They must be completely written before submit_gof / upload_gof / the stage entry points
+ * are called: the library does not wait on the caller's stream (synchronise it first).  They are read on the device after
+ * submit_gof has returned and must stay unmodified until tmc2gpu_wait_inputs returns.                                */
 TMC2_API void*       tmc2gpu_alloc_pinned(size_t bytes);
 TMC2_API void        tmc2gpu_free_pinned(void* p);
 
@@ -219,8 +240,8 @@ TMC2_API void        tmc2gpu_free_pinned(void* p);
  * A GOF is delivered whole or not at all: when submit_gof fails nothing of it is queued; when a launch fails on the
  * device, next_frame reports the error ONCE, drops every frame of that GOF and frees its slot -- the next call
  * continues with the following GOF (or returns TMC2_END).
- * wait_inputs blocks until the host-to-device copies of every GOF submitted so far have finished, i.e. until pinned
- * input planes may be overwritten with the next GOF's samples.                                        */
+ * wait_inputs blocks until the host-to-device copies (device planes: the gather kernel) of every GOF submitted so far have
+ * finished, i.e. until pinned or device input planes may be overwritten with the next GOF's samples.  */
 TMC2_API tmc2_status tmc2gpu_submit_gof(tmc2gpu_ctx* ctx, const tmc2_gof* gof);
 TMC2_API tmc2_status tmc2gpu_wait_inputs(tmc2gpu_ctx* ctx);
 TMC2_API tmc2_status tmc2gpu_next_frame(tmc2gpu_ctx* ctx, tmc2_frame_out* out);

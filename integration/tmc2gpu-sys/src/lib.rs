@@ -83,7 +83,7 @@ pub struct tmc2_gof {
     pub frame_count: u32,
     pub geo_video_frames: u32,
     pub attr_video_frames: u32,
-    pub _reserved: u32,
+    pub input_flags: u32, // TMC2_INPUT_* bits; 0 = every plane in host memory
     pub frames: *const tmc2_frame,
     pub params: tmc2_params,
 }
@@ -131,6 +131,8 @@ extern "C" {
     pub fn tmc2gpu_release_frame(ctx: *mut tmc2gpu_ctx, out: *mut tmc2_frame_out) -> c_int;
     pub fn tmc2gpu_frame_to_ply(ctx: *mut tmc2gpu_ctx, frame: *const tmc2_frame_out, format: u32, dst: *mut c_void, dst_capacity: u64, file_bytes: *mut u64) -> c_int;
 }
+pub const TMC2_INPUT_DEVICE: u32 = 1; // every plane of the GOF is CUDA device memory (NVDEC / ffmpeg CUDA hwaccel)
+pub const TMC2_INPUT_P010: u32 = 2; // 16-bit planes in P010 layout (value in bits 15..6, interleaved UV in attr_u)
 pub const TMC2_PLY_ASCII: u32 = 0;
 pub const TMC2_PLY_BINARY_LE: u32 = 1;
 

@@ -31,6 +31,7 @@ ORIENTATION_REFERENCE, ORIENTATION_SPEC = 0, 1
 CTX_TWO_PASS_SCAN = 1
 CTX_DEVICE_OUTPUT = 2
 LAUNCH_TIMED = 1
+INPUT_DEVICE, INPUT_P010 = 1, 2          # tmc2_gof.input_flags: planes in CUDA device memory / P010 layout
 PLY_ASCII, PLY_BINARY_LE = 0, 1          # tmc2gpu_frame_to_ply formats (src/writer.rs:8-12)
 
 
@@ -84,7 +85,7 @@ class CFrame(C.Structure):
 class CGof(C.Structure):
     _fields_ = [("width", C.c_uint32), ("height", C.c_uint32), ("occ_width", C.c_uint32), ("occ_height", C.c_uint32),
                 ("frame_count", C.c_uint32), ("geo_video_frames", C.c_uint32), ("attr_video_frames", C.c_uint32),
-                ("_reserved", C.c_uint32), ("frames", C.POINTER(CFrame)), ("params", CParams)]
+                ("input_flags", C.c_uint32), ("frames", C.POINTER(CFrame)), ("params", CParams)]
 
 
 class CFrameOut(C.Structure):
@@ -147,13 +148,18 @@ class Params:
 
 @dataclass
 class Gof:
-    """Decoded planes + patch lists of one group of frames, as numpy arrays (tight, C-contiguous).
+    """Decoded planes + patch lists of one group of frames.
 
     occ    [F, occH, occW] u8      reference ``atlas.occ_frames``           (Video<u8>)
     geo    [F, 2, H, W]   u16      reference ``atlas.geo_frames[0]``  frame f*2+m, channel 0
     attr_y [F, 2, H, W]   u16      reference ``atlas.attr_frames[0]`` frame f*2+m, channel 0
     attr_u/attr_v [F, 2, H/2, W/2] u16  channels 1, 2 (4:2:0)
     patches: one PATCH_DTYPE array per frame (``tile.patches``)
+
+    Planes are numpy arrays (host memory) or, all of them, objects exposing ``__cuda_array_interface__`` such as torch
+    CUDA tensors (device memory, ``TMC2_INPUT_DEVICE``; 16-bit planes may be int16 tensors, their bits are read as u16).
+    ``plane_format="p010"`` (device planes only): geo / attr_y samples hold the value in bits 15..6, ``attr_u`` is the
+    interleaved UV array [F, 2, H/2, W] (U first) and ``attr_v`` is None.
     """
     width: int
     height: int
@@ -166,10 +172,12 @@ class Gof:
     params: Params = field(default_factory=Params)
     geo_video_frames: Optional[int] = None
     attr_video_frames: Optional[int] = None
+    plane_format: str = "planar"
 
     @property
     def frame_count(self) -> int:
-        return int(self.occ.shape[0])
+        iface = getattr(self.occ, "__cuda_array_interface__", None)
+        return int(iface["shape"][0] if iface is not None else self.occ.shape[0])
 
     def input_bytes(self) -> int:
         n = self.occ.nbytes + self.geo.nbytes
@@ -185,37 +193,83 @@ class Gof:
                    sel(self.attr_v), [self.patches[i] for i in idx], self.params)
 
 
+class _Plane:
+    """Address arithmetic over a plane array: numpy (host) or ``__cuda_array_interface__`` (device)."""
+
+    def __init__(self, name, a):
+        self.name = name
+        iface = getattr(a, "__cuda_array_interface__", None)
+        self.device = iface is not None
+        if self.device:
+            self.shape = tuple(iface["shape"])
+            self.itemsize = int(iface["typestr"][2:])
+            if iface["typestr"][1] not in "ui":
+                raise ValueError(f"{name}: integer samples expected, got {iface['typestr']}")
+            strides = iface.get("strides")
+            if strides is None:                   # C-contiguous
+                strides, acc = [], self.itemsize
+                for n in reversed(self.shape):
+                    strides.insert(0, acc)
+                    acc *= n
+            self.strides = tuple(strides)
+            self.base = int(iface["data"][0])
+            self.torch_device = getattr(getattr(a, "device", None), "index", None)
+        else:
+            self.shape, self.strides, self.itemsize = a.shape, a.strides, a.itemsize
+            self.base = a.ctypes.data
+
+    def ptr(self, *idx):
+        return self.base + sum(i * s for i, s in zip(idx, self.strides))
+
+    def pitch(self):
+        # rows may be padded (ffmpeg's linesize > width): samples of a row contiguous, row pitch a multiple of the sample size
+        # -- the pitch travels in the *_stride fields (the reference itself assumes tight planes)
+        s, isz = self.strides, self.itemsize
+        if s[-1] != isz or s[-2] % isz or s[-2] < self.shape[-1] * isz:
+            raise ValueError(f"{self.name}: rows must be contiguous runs of samples (row pitch >= width)")
+        return s[-2] // isz
+
+
 class GofView:
     """Builds (and keeps alive) the ``tmc2_gof`` C view of a :class:`Gof`."""
 
     def __init__(self, gof: Gof):
         self.gof = gof
         F = gof.frame_count
-        # planes may be row-padded views (ffmpeg's linesize > width): samples of a row contiguous, row pitch a multiple of
-        # the sample size -- the pitch travels in the *_stride fields (the reference itself assumes tight planes)
-        def pitch(name):
-            a = getattr(gof, name)
-            if a.strides[-1] != a.itemsize or a.strides[-2] % a.itemsize or a.strides[-2] < a.shape[-1] * a.itemsize:
-                raise ValueError(f"{name}: rows must be contiguous runs of samples (row pitch >= width)")
-            return a.strides[-2] // a.itemsize
-        assert gof.occ.dtype == np.uint8 and gof.geo.dtype == np.uint16
+        if gof.plane_format not in ("planar", "p010"):
+            raise ValueError(f"plane_format {gof.plane_format!r}: 'planar' or 'p010'")
+        p010 = gof.plane_format == "p010"
+        names = ["occ", "geo"] + (["attr_y", "attr_u"] + ([] if p010 else ["attr_v"]) if gof.attr_y is not None else [])
+        if p010 and gof.attr_v is not None:
+            raise ValueError("p010: attr_u is the interleaved UV array and attr_v must be None")
+        pl = {n: _Plane(n, getattr(gof, n)) for n in names}
+        on_device = {p.device for p in pl.values()}
+        if len(on_device) > 1:
+            raise ValueError("host (numpy) and device (__cuda_array_interface__) planes mixed in one GOF")
+        self.device_input = on_device == {True}
+        if p010 and not self.device_input:
+            raise ValueError("p010 planes must be device arrays (host P010 is not supported)")
+        if pl["occ"].itemsize != 1 or any(pl[n].itemsize != 2 for n in names[1:]):
+            raise ValueError("occ must hold 8-bit samples, geo / attr_* 16-bit samples")
+        # CUDA devices of the planes, where the producer tells (torch tensors): codec synchronises their current streams
+        self.devices = sorted({p.torch_device for p in pl.values() if self.device_input and p.torch_device is not None})
         self._frames = (CFrame * max(F, 1))()
         self._keep = []
         for f in range(F):
             fr = self._frames[f]
-            fr.occ = gof.occ[f].ctypes.data
-            fr.occ_stride = pitch("occ")
+            fr.occ = pl["occ"].ptr(f)
+            fr.occ_stride = pl["occ"].pitch()
             for m in range(2):
-                fr.geo[m] = gof.geo[f, m].ctypes.data if gof.geo.shape[1] > m else None
+                fr.geo[m] = pl["geo"].ptr(f, m) if pl["geo"].shape[1] > m else None
                 if gof.attr_y is not None:
-                    fr.attr_y[m] = gof.attr_y[f, m].ctypes.data
-                    fr.attr_u[m] = gof.attr_u[f, m].ctypes.data
-                    fr.attr_v[m] = gof.attr_v[f, m].ctypes.data
-            fr.geo_stride = pitch("geo")
+                    fr.attr_y[m] = pl["attr_y"].ptr(f, m)
+                    fr.attr_u[m] = pl["attr_u"].ptr(f, m)
+                    fr.attr_v[m] = None if p010 else pl["attr_v"].ptr(f, m)
+            fr.geo_stride = pl["geo"].pitch()
             if gof.attr_y is not None:
-                fr.attr_stride_y = pitch("attr_y")
-                fr.attr_stride_c = pitch("attr_u")
-                if pitch("attr_v") != fr.attr_stride_c:
+                fr.attr_stride_y = pl["attr_y"].pitch()
+                fr.attr_stride_c = pl["attr_u"].pitch()
+                if not p010 and pl["attr_v"].pitch() != fr.attr_stride_c:
                     raise ValueError("attr_u and attr_v must share one row pitch")
             p = np.ascontiguousarray(gof.patches[f], dtype=PATCH_DTYPE)
             self._keep.append(p)
@@ -223,13 +277,14 @@ class GofView:
             fr.patch_count = len(p)
         g = CGof()
         g.width, g.height = gof.width, gof.height
-        g.occ_height, g.occ_width = gof.occ.shape[1], gof.occ.shape[2]
+        g.occ_height, g.occ_width = pl["occ"].shape[1], pl["occ"].shape[2]
         g.frame_count = F
-        g.geo_video_frames = gof.geo_video_frames if gof.geo_video_frames is not None else F * gof.geo.shape[1]
+        g.geo_video_frames = gof.geo_video_frames if gof.geo_video_frames is not None else F * pl["geo"].shape[1]
         if gof.attr_video_frames is not None:
             g.attr_video_frames = gof.attr_video_frames
         else:
-            g.attr_video_frames = 0 if gof.attr_y is None else F * gof.attr_y.shape[1]
+            g.attr_video_frames = 0 if gof.attr_y is None else F * pl["attr_y"].shape[1]
+        g.input_flags = (INPUT_DEVICE if self.device_input else 0) | (INPUT_P010 if p010 else 0)
         g.frames = C.cast(self._frames, C.POINTER(CFrame))
         g.params = gof.params.to_c()
         self.c = g

@@ -69,12 +69,22 @@ class Context:
             msg = self.lib.tmc2gpu_last_error(self.h)
             raise abi.Tmc2Error(st, where, msg.decode() if msg else "")
 
+    @staticmethod
+    def _inputs_written(view: abi.GofView):
+        """Device planes must be completely written when the library is called (it does not wait on the caller's stream):
+        synchronise torch's current stream on every device that holds planes of the GOF."""
+        if view.device_input and view.devices:
+            import torch
+            for d in view.devices:
+                torch.cuda.current_stream(d).synchronize()
+
     # ---- stage API (one frame, synchronous) -----------------------------------------------------------------
     def generate_block_to_patch_from_occupancy_map_video(self, view: abi.GofView, frame_index: int) -> np.ndarray:
         """src/codec.rs:205-250.  Returns ``block_to_patch`` (patch index + 1, 0 = unowned)."""
         g = view.c
         res = max(g.params.occupancy_resolution, 1)
         out = np.zeros(max((g.width // res) * (g.height // res), 1), dtype=np.uint32)
+        self._inputs_written(view)
         self.check(self.lib.tmc2gpu_generate_block_to_patch_from_occupancy_map_video(
             self.h, view.ref(), frame_index, out.ctypes.data), "generate_block_to_patch_from_occupancy_map_video")
         return out[:(g.width // res) * (g.height // res)]
@@ -98,6 +108,7 @@ class Context:
         bufs["block_to_patch"] = np.zeros(max((g.width // res) * (g.height // res), 1), np.uint32)
         for k, v in bufs.items():
             setattr(o, k, v.ctypes.data)
+        self._inputs_written(view)
         self.check(self.lib.tmc2gpu_generate_point_cloud(self.h, view.ref(), frame_index, C.byref(o)),
                    "generate_point_cloud")
         n = int(o.point_count)
@@ -120,10 +131,12 @@ class Context:
 
     # ---- streaming API: the frame loop src/decoder.rs:188-314 -------------------------------------------------
     def submit_gof(self, view: abi.GofView):
+        self._inputs_written(view)
         self.check(self.lib.tmc2gpu_submit_gof(self.h, view.ref()), "submit_gof")
 
     def wait_inputs(self):
-        """Blocks until the H2D copies of every submitted GOF are done: pinned input planes may be overwritten again."""
+        """Blocks until the inputs of every submitted GOF have been read (H2D copies, or the gather kernel of device planes):
+        pinned or device input planes may be overwritten again."""
         self.check(self.lib.tmc2gpu_wait_inputs(self.h), "wait_inputs")
 
     def next_frame(self, copy: bool = True) -> Optional[PointSet3]:
@@ -203,6 +216,7 @@ class Context:
     # ---- resident path (planes stay in HBM) -------------------------------------------------------------------
     def upload_gof(self, view: abi.GofView) -> "Resident":
         h = C.c_void_p()
+        self._inputs_written(view)
         self.check(self.lib.tmc2gpu_upload_gof(self.h, view.ref(), C.byref(h)), "upload_gof")
         return Resident(self, h, view.c.frame_count)
 

@@ -253,6 +253,28 @@ constexpr int kEmitWarps = TMC2_EMIT_WARPS;                      // warps per CT
 //   geo, attr_y: (x, y, map, frame) box 16 x 16 x 2 x 1      attr_u, attr_v: box 8 x 8 x 2 x 1      occ: (x, y, frame) box 32 x 8 x 1
 struct alignas(64) TileMaps { unsigned long long geo[16], attr_y[16], attr_u[16], attr_v[16], occ[16]; };
 
+// Device-resident input (TMC2_INPUT_DEVICE): one entry per (frame, plane kind, map) of the caller's planes, gathered by
+// ingest_planes_kernel into the batch layout above.  The table travels at the end of the batch's metadata block.
+enum IngestOp : uint32_t {
+  kIngestCopy8 = 0,        // u8 samples, copied
+  kIngestCopy16 = 1,       // u16 samples, copied
+  kIngestShr16 = 2,        // P010 u16 samples: raw >> 6
+  kIngestUv16 = 3,         // P010 interleaved UV pairs: U >> 6 to dst, V >> 6 to dst2
+  kIngestVec = 0x100u,     // flag: source base and pitch are 16-byte aligned -> 16-byte vector loads
+};
+struct alignas(16) IngestPlane {
+  const uint8_t* src;      // caller's plane (this device, or a peer device of the context)
+  uint8_t* dst;            // plane in the batch layout
+  uint8_t* dst2;           // kIngestUv16: the V plane
+  uint32_t spitch;         // source row pitch, bytes
+  uint32_t dpitch;         // destination row pitch, bytes (a multiple of 64)
+  uint32_t rows;
+  uint32_t row_bytes;      // source bytes per row
+  uint32_t op;             // IngestOp (| kIngestVec)
+  uint32_t _pad;
+};
+static_assert(sizeof(IngestPlane) == 48, "IngestPlane is three 16-byte vectors");
+
 // launch wrappers (kernels.cu); every one enqueues on `stream` and returns the cudaGetLastError() code
 int launch_block_to_patch(const UnpackArgs& a, uint32_t n_slots, void* stream);
 int launch_compact_owned(const UnpackArgs& a, void* stream);   // after block_to_patch: per-frame list of owned slots
@@ -266,6 +288,8 @@ int launch_smooth_filter(const UnpackArgs& a, void* stream);   // boundary point
 int launch_smooth_clear(const UnpackArgs& a, void* stream);    // reset touched cells (+ keys) of the group
 int launch_yuv_to_rgb_flat(const uint16_t* yuv, uint8_t* rgb, uint64_t n, void* stream);
 int launch_fill_u32(uint32_t* p, uint64_t n, uint32_t v, void* stream);
+// every plane of `table` (device memory, n_planes entries); max_rows / max_row_bytes over the table size the grid
+int launch_ingest_planes(const IngestPlane* table, uint32_t n_planes, uint32_t max_rows, uint32_t max_row_bytes, void* stream);
 int kernel_launch_count_reset();   // returns launches since the last reset
 
 // ply.cu: a frame in HBM formatted as the body of a PLY file (src/writer.rs:62-75).  measure -> scan -> write for the ASCII

@@ -1983,6 +1983,82 @@ __global__ void __launch_bounds__(256) fill_u32_kernel(uint32_t* p, uint64_t n, 
 }
 
 // ----------------------------------------------------------------------------------------------------------------
+// ingest_planes_kernel: the caller's device-resident planes (TMC2_INPUT_DEVICE) -> batch layout.  CTA = (row range,
+// plane); thread = one 16-byte chunk of a source row at a time, four chunks loaded before any is stored.  A chunk takes
+// the vector path when the plane's base and pitch are 16-byte aligned (decided on the host) and the chunk is whole; the
+// rest of a row and every chunk of an unaligned plane go sample by sample.  Destination rows are 64-element aligned.
+// ----------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t p010_pair(uint32_t w) { return (w >> 6) & 0x03FF03FFu; }   // two samples, raw >> 6
+
+__device__ __forceinline__ void ingest_store_vec(const IngestPlane& p, uint32_t op, uint32_t r, uint32_t c, uint4 v) {
+  if (op == kIngestUv16) {                 // u0 v0 u1 v1 | u2 v2 u3 v3 -> u0 u1 u2 u3, v0 v1 v2 v3
+    const uint2 u = make_uint2(p010_pair(__byte_perm(v.x, v.y, 0x5410)), p010_pair(__byte_perm(v.z, v.w, 0x5410)));
+    const uint2 w = make_uint2(p010_pair(__byte_perm(v.x, v.y, 0x7632)), p010_pair(__byte_perm(v.z, v.w, 0x7632)));
+    *reinterpret_cast<uint2*>(p.dst + (size_t)r * p.dpitch + c * 8) = u;
+    *reinterpret_cast<uint2*>(p.dst2 + (size_t)r * p.dpitch + c * 8) = w;
+    return;
+  }
+  if (op == kIngestShr16) v = make_uint4(p010_pair(v.x), p010_pair(v.y), p010_pair(v.z), p010_pair(v.w));
+  *reinterpret_cast<uint4*>(p.dst + (size_t)r * p.dpitch + c * 16) = v;
+}
+
+__device__ __forceinline__ void ingest_narrow(const IngestPlane& p, uint32_t op, uint32_t r, uint32_t c, uint32_t n) {
+  const uint8_t* s = p.src + (size_t)r * p.spitch + c * 16;
+  if (op == kIngestCopy8) {
+    uint8_t* d = p.dst + (size_t)r * p.dpitch + c * 16;
+    for (uint32_t j = 0; j < n; ++j) d[j] = __ldg(s + j);
+  } else if (op == kIngestUv16) {
+    const uint16_t* s16 = reinterpret_cast<const uint16_t*>(s);
+    uint16_t* du = reinterpret_cast<uint16_t*>(p.dst + (size_t)r * p.dpitch) + c * 4;
+    uint16_t* dv = reinterpret_cast<uint16_t*>(p.dst2 + (size_t)r * p.dpitch) + c * 4;
+    for (uint32_t j = 0; j < n / 4; ++j) {
+      du[j] = (uint16_t)(__ldg(s16 + 2 * j) >> 6);
+      dv[j] = (uint16_t)(__ldg(s16 + 2 * j + 1) >> 6);
+    }
+  } else {
+    const uint16_t* s16 = reinterpret_cast<const uint16_t*>(s);
+    uint16_t* d = reinterpret_cast<uint16_t*>(p.dst + (size_t)r * p.dpitch + c * 16);
+    const uint32_t sh = op == kIngestShr16 ? 6u : 0u;
+    for (uint32_t j = 0; j < n / 2; ++j) d[j] = (uint16_t)(__ldg(s16 + j) >> sh);
+  }
+}
+
+constexpr uint32_t kIngestThreads = 256, kIngestUnroll = 4;
+
+__global__ void __launch_bounds__(kIngestThreads) ingest_planes_kernel(const IngestPlane* __restrict__ table, uint32_t n_planes,
+                                                                     uint32_t rows_per_cta) {
+  for (uint32_t pi = blockIdx.y; pi < n_planes; pi += gridDim.y) {
+    const IngestPlane p = table[pi];
+    const uint32_t r0 = blockIdx.x * rows_per_cta;
+    if (r0 >= p.rows) continue;
+    const uint32_t rows = min(p.rows - r0, rows_per_cta);
+    const uint32_t nch = (p.row_bytes + 15u) >> 4;
+    const uint32_t total = rows * nch;
+    const uint32_t op = p.op & 0xFFu;
+    const bool vec = (p.op & kIngestVec) != 0;
+    for (uint32_t i0 = threadIdx.x; i0 < total; i0 += kIngestUnroll * kIngestThreads) {
+      uint4 v[kIngestUnroll];
+#pragma unroll
+      for (uint32_t k = 0; k < kIngestUnroll; ++k) {
+        const uint32_t i = i0 + k * kIngestThreads;
+        const uint32_t r = r0 + i / nch, c = i % nch;
+        v[k] = make_uint4(0, 0, 0, 0);
+        if (vec && i < total && c * 16 + 16 <= p.row_bytes) v[k] = ldg_nc_v4(p.src + (size_t)r * p.spitch + c * 16);
+      }
+#pragma unroll
+      for (uint32_t k = 0; k < kIngestUnroll; ++k) {
+        const uint32_t i = i0 + k * kIngestThreads;
+        if (i >= total) break;
+        const uint32_t r = r0 + i / nch, c = i % nch;
+        const uint32_t n = min(16u, p.row_bytes - c * 16);
+        if (vec && n == 16) ingest_store_vec(p, op, r, c, v[k]);
+        else ingest_narrow(p, op, r, c, n);
+      }
+    }
+  }
+}
+
+// ----------------------------------------------------------------------------------------------------------------
 // launch wrappers
 // ----------------------------------------------------------------------------------------------------------------
 static inline int after_launch() { ++g_launches; return (int)cudaGetLastError(); }
@@ -2085,6 +2161,15 @@ int launch_yuv_to_rgb_flat(const uint16_t* yuv, uint8_t* rgb, uint64_t n, void* 
 int launch_fill_u32(uint32_t* p, uint64_t n, uint32_t v, void* stream) {
   if (n == 0) return 0;
   fill_u32_kernel<<<148 * 8, 256, 0, (cudaStream_t)stream>>>(p, n, v);
+  return after_launch();
+}
+
+int launch_ingest_planes(const IngestPlane* table, uint32_t n_planes, uint32_t max_rows, uint32_t max_row_bytes, void* stream) {
+  if (n_planes == 0 || max_rows == 0 || max_row_bytes == 0) return 0;
+  // ~64 KB of source per CTA: enough work per CTA to amortise its start, enough CTAs to fill 148 SMs several times over
+  const uint32_t rows_per_cta = std::max(1u, (64u << 10) / max_row_bytes);
+  const dim3 grid((max_rows + rows_per_cta - 1) / rows_per_cta, std::min(n_planes, 65535u));
+  ingest_planes_kernel<<<grid, kIngestThreads, 0, (cudaStream_t)stream>>>(table, n_planes, rows_per_cta);
   return after_launch();
 }
 

@@ -230,6 +230,21 @@ static bool encode_map(unsigned long long* out, void* base, uint32_t esz, uint32
   return true;
 }
 
+// Allocation that holds a device pointer (cuMemGetAddressRange, reached the same way).
+typedef CUresult (*AddressRangeFn)(CUdeviceptr*, size_t*, CUdeviceptr);
+static AddressRangeFn address_range_fn() {
+  static AddressRangeFn fn = [] {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuMemGetAddressRange", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
+      cudaGetLastError();
+      p = nullptr;
+    }
+    return (AddressRangeFn)p;
+  }();
+  return fn;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // validation: everything the reference asserts / unwraps / leaves unimplemented on this path
 // ---------------------------------------------------------------------------------------------------------------
@@ -287,12 +302,60 @@ static tmc2_status validate_params(const tmc2_gof* g, Err& err) {
       if ((maxs + P.cgrid_size - 1) / P.cgrid_size > 1024) FAIL(TMC2_ERR_UNSUPPORTED, "colour grid wider than 1024 cells");
     }
   }
+  if (g->input_flags & ~(TMC2_INPUT_DEVICE | TMC2_INPUT_P010))
+    FAIL(TMC2_ERR_INVALID_ARG, "input_flags 0x%x: unknown bits", g->input_flags);
+  if ((g->input_flags & TMC2_INPUT_P010) && !(g->input_flags & TMC2_INPUT_DEVICE))
+    FAIL(TMC2_ERR_UNSUPPORTED, "TMC2_INPUT_P010 is only accepted with TMC2_INPUT_DEVICE (host P010 planes are not supported)");
   return TMC2_OK;
 }
 
-static tmc2_status validate_frame(const tmc2_gof* g, uint32_t f, Err& err) {
+// Device planes (TMC2_INPUT_DEVICE): the allocations they were found in, with their devices.  A plane inside an allocation
+// already seen costs no driver call (a GOF held in one tensor is checked with one query per plane kind).
+struct DevRange { uintptr_t base; size_t size; int device; };
+
+static tmc2_status check_device_plane(const void* p, uint32_t rows, size_t pitch_bytes, size_t row_bytes, const std::vector<int>& devices,
+                                      std::vector<DevRange>& ranges, uint32_t f, const char* what, Err& err) {
+  const uintptr_t a = (uintptr_t)p;
+  const size_t extent = (size_t)(rows - 1) * pitch_bytes + row_bytes;
+  for (const DevRange& r : ranges)
+    if (a >= r.base && a - r.base < r.size) {
+      if (extent > r.size - (a - r.base))
+        FAIL(TMC2_ERR_INVALID_ARG, "frame %u: %s plane (%zu bytes from its start) runs past the end of its allocation", f, what, extent);
+      return TMC2_OK;
+    }
+  cudaPointerAttributes at{};
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+    cudaGetLastError();
+    FAIL(TMC2_ERR_INVALID_ARG, "frame %u: %s plane is not CUDA device memory (TMC2_INPUT_DEVICE)", f, what);
+  }
+  if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged)
+    FAIL(TMC2_ERR_INVALID_ARG, "frame %u: %s plane is host memory, TMC2_INPUT_DEVICE wants device memory", f, what);
+  if (std::find(devices.begin(), devices.end(), at.device) == devices.end())
+    FAIL(TMC2_ERR_INVALID_ARG, "frame %u: %s plane is on device %d, which is not a device of the context", f, what, at.device);
+  AddressRangeFn fn = address_range_fn();
+  if (!fn) FAIL(TMC2_ERR_CUDA, "cuMemGetAddressRange is not available from the driver");
+  int cur = 0;
+  if (cudaGetDevice(&cur) != cudaSuccess || cudaSetDevice(at.device) != cudaSuccess) {
+    cudaGetLastError();
+    FAIL(TMC2_ERR_CUDA, "cudaSetDevice(%d) failed while checking a device plane", at.device);
+  }
+  CUdeviceptr base = 0;
+  size_t size = 0;
+  const CUresult cr = fn(&base, &size, (CUdeviceptr)a);
+  cudaSetDevice(cur);
+  if (cr != CUDA_SUCCESS) FAIL(TMC2_ERR_INVALID_ARG, "frame %u: %s plane: no device allocation holds it (CUresult %d)", f, what, (int)cr);
+  ranges.push_back({(uintptr_t)base, size, at.device});
+  if (extent > size - (a - (uintptr_t)base))
+    FAIL(TMC2_ERR_INVALID_ARG, "frame %u: %s plane (%zu bytes from its start) runs past the end of its allocation", f, what, extent);
+  return TMC2_OK;
+}
+
+// `devices` / `ranges`: the context's devices and the allocations of the GOF's device planes seen so far (TMC2_INPUT_DEVICE)
+static tmc2_status validate_frame(const tmc2_gof* g, uint32_t f, const std::vector<int>& devices, std::vector<DevRange>& ranges,
+                                  Err& err) {
   const tmc2_params& P = g->params;
   const tmc2_frame& fr = g->frames[f];
+  const bool p010 = (g->input_flags & TMC2_INPUT_P010) != 0;
   // codec.rs:318-320: geometry video must hold frames f*M .. f*M+M-1
   if ((uint64_t)g->geo_video_frames < (uint64_t)f * 2 + 2)
     FAIL(TMC2_ERR_SHORT_VIDEO, "geometry video has %u frames, frame %u needs %llu (codec.rs:318)", g->geo_video_frames, f,
@@ -301,10 +364,14 @@ static tmc2_status validate_frame(const tmc2_gof* g, uint32_t f, Err& err) {
     FAIL(TMC2_ERR_SHORT_VIDEO, "attribute video has %u frames, frame %u needs %llu (codec.rs:589,637)",
          g->attr_video_frames, f, (unsigned long long)f * 2 + 2);
   if (!fr.occ || !fr.geo[0] || !fr.geo[1]) FAIL(TMC2_ERR_INVALID_ARG, "frame %u: NULL occupancy / geometry plane", f);
-  if (P.attribute_count && (!fr.attr_y[0] || !fr.attr_y[1] || !fr.attr_u[0] || !fr.attr_u[1] || !fr.attr_v[0] || !fr.attr_v[1]))
+  if (P.attribute_count && (!fr.attr_y[0] || !fr.attr_y[1] || !fr.attr_u[0] || !fr.attr_u[1] ||
+                            (!p010 && (!fr.attr_v[0] || !fr.attr_v[1]))))
     FAIL(TMC2_ERR_INVALID_ARG, "frame %u: NULL attribute plane", f);
+  if (P.attribute_count && p010 && (fr.attr_v[0] || fr.attr_v[1]))
+    FAIL(TMC2_ERR_INVALID_ARG, "frame %u: attr_v must be NULL with TMC2_INPUT_P010 (attr_u is the interleaved UV plane)", f);
+  // P010: attr_u rows hold width/2 interleaved (U, V) pairs = width elements
   if (fr.occ_stride < g->occ_width || fr.geo_stride < g->width ||
-      (P.attribute_count && (fr.attr_stride_y < g->width || fr.attr_stride_c < g->width / 2)))
+      (P.attribute_count && (fr.attr_stride_y < g->width || fr.attr_stride_c < (p010 ? g->width : g->width / 2))))
     FAIL(TMC2_ERR_INVALID_ARG, "frame %u: stride smaller than width", f);
   if (fr.patch_count && !fr.patches) FAIL(TMC2_ERR_INVALID_ARG, "frame %u: NULL patch list", f);
   if (fr.patch_count > 65535) FAIL(TMC2_ERR_CAPACITY, "frame %u: more than 65535 patches", f);
@@ -338,6 +405,23 @@ static tmc2_status validate_frame(const tmc2_gof* g, uint32_t f, Err& err) {
       if (x < 0 || y < 0 || x >= (int64_t)g->width || y >= (int64_t)g->height)
         FAIL(TMC2_ERR_PATCH_OUT_OF_CANVAS, "frame %u patch %u: pixel (%lld,%lld) outside the canvas (decoder.rs:848)", f, i,
              (long long)x, (long long)y);
+    }
+  }
+  if (g->input_flags & TMC2_INPUT_DEVICE) {
+    if (check_device_plane(fr.occ, g->occ_height, fr.occ_stride, g->occ_width, devices, ranges, f, "occupancy", err)) return err.st;
+    for (int m = 0; m < 2; ++m)
+      if (check_device_plane(fr.geo[m], g->height, (size_t)fr.geo_stride * 2, (size_t)g->width * 2, devices, ranges, f, "geometry", err))
+        return err.st;
+    if (P.attribute_count) {
+      const uint32_t hc = g->height / 2;
+      for (int m = 0; m < 2; ++m) {
+        if (check_device_plane(fr.attr_y[m], g->height, (size_t)fr.attr_stride_y * 2, (size_t)g->width * 2, devices, ranges, f,
+                               "attribute Y", err)) return err.st;
+        if (check_device_plane(fr.attr_u[m], hc, (size_t)fr.attr_stride_c * 2, (size_t)(p010 ? g->width : g->width / 2) * 2, devices,
+                               ranges, f, p010 ? "attribute UV" : "attribute U", err)) return err.st;
+        if (!p010 && check_device_plane(fr.attr_v[m], hc, (size_t)fr.attr_stride_c * 2, (size_t)(g->width / 2) * 2, devices, ranges, f,
+                                        "attribute V", err)) return err.st;
+      }
     }
   }
   return TMC2_OK;
@@ -388,7 +472,10 @@ struct Batch {
   std::vector<cudaEvent_t> ev_grp;    // 2 per group: around the unpack launch
   PinBuf h_in, h_meta, h_small, h_out, h_ply;
   DevBuf d_ply, d_ply_sums;           // tmc2gpu_frame_to_ply: body scratch, block sums + offsets + total
-  size_t meta_patch_off = 0, meta_slot_off = 0, meta_tf_off = 0, meta_ftb_off = 0, meta_bytes = 0;
+  size_t meta_patch_off = 0, meta_slot_off = 0, meta_tf_off = 0, meta_ftb_off = 0, meta_ingest_off = 0, meta_bytes = 0;
+  uint32_t input_flags = 0;           // tmc2_gof.input_flags of the loaded GOF
+  uint32_t n_ingest = 0;              // device planes: entries of the ingest table (end of the metadata block)
+  uint32_t ingest_launches = 0;       // ingest kernel launched by upload(), counted with the next launch()
 
   cudaEvent_t ev[8] = {};             // stage boundaries: 0 start,1 after b2p,2 after unpack,3 geo,4 col,5 rgb
   cudaEvent_t ev_counts = nullptr, ev_inputs_free = nullptr;
@@ -466,6 +553,7 @@ struct Batch {
     res = params.occupancy_resolution; prec = params.occupancy_precision;
     bw = W / res; bh = H / res;
     want = want_flags;
+    input_flags = g->input_flags;
     Hc = H / 2;
     geo_pitch = round_up(W, 64); attr_pitch_y = round_up(W, 64); attr_pitch_c = round_up(std::max(W / 2, 1u), 64);
     occ_pitch = round_up(occ_w, 16);
@@ -534,7 +622,10 @@ struct Batch {
     meta_slot_off = round_up64(h_patches.size() * sizeof(DevPatch), 256);
     meta_tf_off = meta_slot_off + round_up64((uint64_t)n_slots * sizeof(SlotRec), 256);
     meta_ftb_off = meta_tf_off + round_up64((uint64_t)n_tiles * 4, 256);
-    meta_bytes = meta_ftb_off + round_up64((uint64_t)(F + 1) * 4, 256);
+    meta_ingest_off = meta_ftb_off + round_up64((uint64_t)(F + 1) * 4, 256);
+    // one table entry per (frame, kind, map): occupancy, 2 geometry, 2 luma, 2 UV (P010) or 2 U + 2 V
+    n_ingest = (input_flags & TMC2_INPUT_DEVICE) ? F * (3 + (attr ? ((input_flags & TMC2_INPUT_P010) ? 4 : 6) : 0)) : 0;
+    meta_bytes = meta_ingest_off + (size_t)n_ingest * sizeof(IngestPlane);
     CU(d_meta.ensure(meta_bytes));
     CU(h_meta.ensure(meta_bytes));
     CU(d_b2p.ensure(std::max<size_t>((size_t)F * bw * bh * 4, 4)));
@@ -675,8 +766,10 @@ struct Batch {
     }
   }
 
-  tmc2_status upload(const tmc2_gof* g, uint32_t first, Err& err, bool use_pool = true) {
+  // dev_ranges: allocations of the GOF's device planes (validate_frame), for TMC2_INPUT_DEVICE
+  tmc2_status upload(const tmc2_gof* g, uint32_t first, const std::vector<DevRange>& dev_ranges, Err& err, bool use_pool = true) {
     CU(cudaSetDevice(device));
+    if (input_flags & TMC2_INPUT_DEVICE) return upload_device(g, first, dev_ranges, err);
     const bool attr = params.attribute_count != 0;
     std::vector<Seg> segs;
     size_t stage_bytes = 0;
@@ -743,13 +836,73 @@ struct Batch {
       i = j;
     }
     CU(flush());
-    // metadata
+    if (send_meta(err)) return err.st;
+    CU(cudaEventRecord(ev_inputs_free, stream));
+    return TMC2_OK;
+  }
+
+  // metadata block (patches, slots, tile -> frame, frame tile ranges; the ingest table is already in place) -> d_meta
+  tmc2_status send_meta(Err& err) {
     uint8_t* m = h_meta.as<uint8_t>();
     if (!h_patches.empty()) memcpy(m + meta_patch_off, h_patches.data(), h_patches.size() * sizeof(DevPatch));
     if (n_slots) memcpy(m + meta_slot_off, h_slot_rec.data(), (size_t)n_slots * sizeof(SlotRec));
     if (n_tiles) memcpy(m + meta_tf_off, h_tile_frame.data(), (size_t)n_tiles * 4);
     memcpy(m + meta_ftb_off, h_ftb.data(), (size_t)(F + 1) * 4);
     CU(cudaMemcpyAsync(d_meta.p, m, meta_bytes, cudaMemcpyHostToDevice, stream));
+    return TMC2_OK;
+  }
+
+  // TMC2_INPUT_DEVICE: no staging and no H2D of planes.  The planes' table goes with the metadata, and one kernel gathers
+  // every plane into the batch layout (the same layout the host path produces, so everything downstream is unchanged).
+  tmc2_status upload_device(const tmc2_gof* g, uint32_t first, const std::vector<DevRange>& dev_ranges, Err& err) {
+    for (const DevRange& r : dev_ranges) {
+      if (r.device == device) continue;
+      int can = 0;
+      CU(cudaDeviceCanAccessPeer(&can, device, r.device));
+      if (!can) FAIL(TMC2_ERR_UNSUPPORTED, "device %d cannot read input planes on device %d (no peer access between them)", device, r.device);
+      const cudaError_t e = cudaDeviceEnablePeerAccess(r.device, 0);
+      if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+      else CU(e);
+    }
+    // the previous GOF of this batch must have been read (ingest done, metadata copied) before its table is written again
+    CU(cudaEventSynchronize(ev_inputs_free));
+    const bool attr = params.attribute_count != 0, p010 = (input_flags & TMC2_INPUT_P010) != 0;
+    IngestPlane* tab = reinterpret_cast<IngestPlane*>(h_meta.as<uint8_t>() + meta_ingest_off);
+    uint32_t n = 0, max_rows = 0, max_row_bytes = 0;
+    auto add = [&](const void* src, size_t spitch, uint32_t rows, uint32_t row_bytes, uint8_t* dst, uint8_t* dst2, uint32_t dpitch,
+                   uint32_t op) {
+      IngestPlane& e = tab[n++];
+      e.src = static_cast<const uint8_t*>(src); e.dst = dst; e.dst2 = dst2;
+      e.spitch = (uint32_t)spitch; e.dpitch = dpitch; e.rows = rows; e.row_bytes = row_bytes;
+      e.op = op | (((uintptr_t)src % 16 == 0 && spitch % 16 == 0) ? (uint32_t)kIngestVec : 0u);
+      e._pad = 0;
+      max_rows = std::max(max_rows, rows); max_row_bytes = std::max(max_row_bytes, row_bytes);
+    };
+    const uint32_t op16 = p010 ? kIngestShr16 : kIngestCopy16;
+    const size_t occ_plane = (size_t)occ_h * occ_pitch, geo_plane = (size_t)H * geo_pitch * 2, y_plane = (size_t)H * attr_pitch_y * 2;
+    const size_t c_plane = (size_t)std::max(Hc, 1u) * attr_pitch_c * 2;
+    for (uint32_t k = 0; k < F; ++k) {
+      const tmc2_frame& fr = g->frames[first + k];
+      add(fr.occ, fr.occ_stride, occ_h, occ_w, d_occ.as<uint8_t>() + k * occ_plane, nullptr, occ_pitch, kIngestCopy8);
+      for (uint32_t m = 0; m < 2; ++m) {
+        const size_t km = (size_t)k * 2 + m;
+        add(fr.geo[m], (size_t)fr.geo_stride * 2, H, W * 2, d_geo.as<uint8_t>() + km * geo_plane, nullptr, geo_pitch * 2, op16);
+        if (!attr) continue;
+        add(fr.attr_y[m], (size_t)fr.attr_stride_y * 2, H, W * 2, d_ay.as<uint8_t>() + km * y_plane, nullptr, attr_pitch_y * 2, op16);
+        if (p010) {
+          add(fr.attr_u[m], (size_t)fr.attr_stride_c * 2, Hc, W * 2, d_au.as<uint8_t>() + km * c_plane, d_av.as<uint8_t>() + km * c_plane,
+              attr_pitch_c * 2, kIngestUv16);
+        } else {
+          add(fr.attr_u[m], (size_t)fr.attr_stride_c * 2, Hc, (W / 2) * 2, d_au.as<uint8_t>() + km * c_plane, nullptr, attr_pitch_c * 2, op16);
+          add(fr.attr_v[m], (size_t)fr.attr_stride_c * 2, Hc, (W / 2) * 2, d_av.as<uint8_t>() + km * c_plane, nullptr, attr_pitch_c * 2, op16);
+        }
+      }
+    }
+    if (n != n_ingest) FAIL(TMC2_ERR_INTERNAL, "ingest table: %u entries, %u expected", n, n_ingest);
+    if (send_meta(err)) return err.st;
+    KL(launch_ingest_planes(reinterpret_cast<const IngestPlane*>(d_meta.as<uint8_t>() + meta_ingest_off), n, max_rows, max_row_bytes,
+                            stream));
+    ingest_launches = 1;
     CU(cudaEventRecord(ev_inputs_free, stream));
     return TMC2_OK;
   }
@@ -966,7 +1119,8 @@ struct Batch {
       if (a.out.yuv) CU(cudaMemcpyAsync(d_yuv_pre.p, d_yuv.p, (size_t)F * cap * 6, cudaMemcpyDeviceToDevice, s));
     }
     if (timed) CU(cudaEventRecord(ev[3], s)); if (timed) CU(cudaEventRecord(ev[4], s)); if (timed) CU(cudaEventRecord(ev[5], s));
-    launches = (uint32_t)kernel_launch_count_reset();
+    launches = (uint32_t)kernel_launch_count_reset() + ingest_launches;
+    ingest_launches = 0;
     counts_ready = false; outputs_enqueued = false; counts_enqueued = false;
     return TMC2_OK;
   }
@@ -1199,8 +1353,9 @@ tmc2_status tmc2gpu_submit_gof(tmc2gpu_ctx* ctx, const tmc2_gof* gof) {
       (ctx->limits.max_height && gof->height > ctx->limits.max_height)) {
     err.st = TMC2_ERR_CAPACITY; err.msg = "frame larger than limits.max_width/height"; return ctx->fail();
   }
+  std::vector<DevRange> dev_ranges;
   for (uint32_t f = 0; f < gof->frame_count; ++f)
-    if (validate_frame(gof, f, err)) return ctx->fail();
+    if (validate_frame(gof, f, ctx->devices, dev_ranges, err)) return ctx->fail();
   if (gof->frame_count == 0) return TMC2_OK;
 
   // Frame-wise sharding: contiguous slices of the GOF, one per device; no collective (SURVEY.md 8e).  A device's slice can
@@ -1266,7 +1421,7 @@ tmc2_status tmc2gpu_submit_gof(tmc2gpu_ctx* ctx, const tmc2_gof* gof) {
     TraceClock pt;
     if (b->prepare(gof, pc.lo, pc.hi - pc.lo, 0, e)) return;
     const double t_prep = pt.lap();
-    if (b->upload(gof, pc.lo, e, pieces.size() == 1)) return;
+    if (b->upload(gof, pc.lo, dev_ranges, e, pieces.size() == 1)) return;
     const double t_up = pt.lap();
     if (b->launch(b->stream, e)) return;
     if (b->enqueue_counts(b->stream, e)) return;          // counts travel right behind the kernels
@@ -1494,12 +1649,13 @@ tmc2_status tmc2gpu_upload_gof(tmc2gpu_ctx* ctx, const tmc2_gof* gof, tmc2_resid
   Err& err = ctx->err;
   err = Err();
   if (validate_params(gof, err)) return ctx->fail();
+  std::vector<DevRange> dev_ranges;
   for (uint32_t f = 0; f < gof->frame_count; ++f)
-    if (validate_frame(gof, f, err)) return ctx->fail();
+    if (validate_frame(gof, f, ctx->devices, dev_ranges, err)) return ctx->fail();
   std::unique_ptr<tmc2_resident> r(new tmc2_resident());
   r->batch.reset(new Batch());
   Batch* b = r->batch.get();
-  if (b->init(ctx->devices[0], ctx->two_pass, err) || b->prepare(gof, 0, gof->frame_count, 0, err) || b->upload(gof, 0, err))
+  if (b->init(ctx->devices[0], ctx->two_pass, err) || b->prepare(gof, 0, gof->frame_count, 0, err) || b->upload(gof, 0, dev_ranges, err))
     return ctx->fail();
   if (cudaStreamSynchronize(b->stream) != cudaSuccess) { err.st = TMC2_ERR_CUDA; err.msg = "upload sync"; return ctx->fail(); }
   b->h_in.release();   // planes now live in HBM; the staging area is not needed again
@@ -1643,9 +1799,11 @@ static tmc2_status run_single(tmc2gpu_ctx* ctx, const tmc2_gof* gof, uint32_t fr
   err = Err();
   if (validate_params(gof, err)) return err.st;
   if (frame_index >= gof->frame_count) FAIL(TMC2_ERR_INVALID_ARG, "frame_index %u >= frame_count %u", frame_index, gof->frame_count);
-  if (validate_frame(gof, frame_index, err)) return err.st;
+  std::vector<DevRange> dev_ranges;
+  if (validate_frame(gof, frame_index, ctx->devices, dev_ranges, err)) return err.st;
   Batch* b = ctx->stage_batch.get();
-  if (b->prepare(gof, frame_index, 1, want, err) || b->upload(gof, frame_index, err) || b->launch(b->stream, err)) return err.st;
+  if (b->prepare(gof, frame_index, 1, want, err) || b->upload(gof, frame_index, dev_ranges, err) || b->launch(b->stream, err))
+    return err.st;
   if (b->fetch_counts(b->stream, err)) return err.st;
   ctx->last_batch = b;
   return TMC2_OK;

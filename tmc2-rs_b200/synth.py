@@ -284,3 +284,39 @@ def kat_appendix_c() -> Gof:
     patches[0] = (0, 0, 1, 1, 100, 200, 16, 1, 1, 0, 2, 1, 0, ORIENT_DEFAULT, 0, (0, 0))
     patches[1] = (1, 0, 1, 1, 10, 20, 1024 - 64, 1, 1, 1, 2, 0, 1, ORIENT_SWAP, 0, (0, 0))
     return Gof(W, H, occ, geo, ay, au, av, [patches], Params())
+
+
+def to_device(gof: Gof, device, pad: int = 0, p010: bool = False, seed: int = 0, offset: int = 0) -> Gof:
+    """Device copy of a host GOF as torch CUDA tensors, the way a GPU video decoder would hand its planes over.
+
+    pad: extra samples at the end of every row (row pitch = width + pad); offset: the planes start `offset` samples into
+    their allocation (a base address that is not 16-byte aligned).  p010: 16-bit samples become ``v << 6`` with seeded noise
+    in the low 6 bits, and U / V are interleaved into one [F, 2, H/2, W] plane (NVDEC / ffmpeg ``p010le``); 16-bit planes
+    are int16 tensors (torch has no full uint16 support), read bit for bit as u16."""
+    import torch
+    gen = torch.Generator(device=device)
+    gen.manual_seed(seed)
+
+    def put(a: np.ndarray, shift: bool):
+        lead, w = a.shape[:-1], a.shape[-1]
+        n = int(np.prod(lead)) * (w + pad)
+        store = torch.zeros(n + offset, dtype=torch.int16 if a.itemsize == 2 else torch.uint8, device=device)
+        t = store[offset:].view(*lead, w + pad)[..., :w]
+        host = a.view(np.int16) if a.itemsize == 2 else a
+        if shift:
+            host = (a.astype(np.uint16) << 6).view(np.int16)
+        t.copy_(torch.from_numpy(np.ascontiguousarray(host)).to(device))
+        if shift:
+            t |= torch.randint(0, 64, t.shape, generator=gen, device=device, dtype=torch.int16)
+        return t
+
+    if gof.attr_y is None:
+        ay = au = av = None
+    elif p010:
+        uv = np.empty(gof.attr_u.shape[:-1] + (2 * gof.attr_u.shape[-1],), np.uint16)
+        uv[..., 0::2], uv[..., 1::2] = gof.attr_u, gof.attr_v
+        ay, au, av = put(gof.attr_y, True), put(uv, True), None
+    else:
+        ay, au, av = put(gof.attr_y, False), put(gof.attr_u, False), put(gof.attr_v, False)
+    return Gof(gof.width, gof.height, put(gof.occ, False), put(gof.geo, p010), ay, au, av, gof.patches, gof.params,
+               gof.geo_video_frames, gof.attr_video_frames, "p010" if p010 else "planar")
