@@ -309,14 +309,55 @@ static tmc2_status validate_params(const tmc2_gof* g, Err& err) {
   return TMC2_OK;
 }
 
+// The five plane kinds, in the order of the batch layout (device_types.h)
+enum PlaneKind : uint32_t { kOcc, kGeo, kAttrY, kAttrU, kAttrV, kPlaneKinds };
+
+// One plane of a frame as the caller holds it
+struct SrcPlane {
+  uint32_t kind, map;
+  const uint8_t* p;
+  size_t pitch;                        // bytes
+  uint32_t rows;
+  size_t row_bytes;
+  const char* name;                    // in messages
+  size_t extent() const { return (size_t)(rows - 1) * pitch + row_bytes; }   // bytes from p to the end of the last row
+};
+constexpr uint32_t kMaxFramePlanes = 9;
+
+// The planes of frame f as the caller holds them: occupancy, the two geometry maps, then attribute Y, U, V of map 0 and of
+// map 1.  Under TMC2_INPUT_P010 attr_u is the interleaved UV plane (W/2 (U, V) pairs = W samples a row) and there is no V plane.
+static uint32_t frame_planes(const tmc2_gof* g, uint32_t f, SrcPlane (&out)[kMaxFramePlanes]) {
+  const tmc2_frame& fr = g->frames[f];
+  const bool p010 = (g->input_flags & TMC2_INPUT_P010) != 0;
+  const uint32_t W = g->width, H = g->height;
+  uint32_t n = 0;
+  auto add = [&](uint32_t kind, uint32_t m, const void* p, uint32_t stride, uint32_t esz, uint32_t rows, uint32_t width, const char* name) {
+    out[n++] = {kind, m, static_cast<const uint8_t*>(p), (size_t)stride * esz, rows, (size_t)width * esz, name};
+  };
+  add(kOcc, 0, fr.occ, fr.occ_stride, 1, g->occ_height, g->occ_width, "occupancy");
+  for (uint32_t m = 0; m < 2; ++m) add(kGeo, m, fr.geo[m], fr.geo_stride, 2, H, W, "geometry");
+  if (g->params.attribute_count)
+    for (uint32_t m = 0; m < 2; ++m) {
+      add(kAttrY, m, fr.attr_y[m], fr.attr_stride_y, 2, H, W, "attribute Y");
+      if (p010) {
+        add(kAttrU, m, fr.attr_u[m], fr.attr_stride_c, 2, H / 2, W, "attribute UV");
+      } else {
+        add(kAttrU, m, fr.attr_u[m], fr.attr_stride_c, 2, H / 2, W / 2, "attribute U");
+        add(kAttrV, m, fr.attr_v[m], fr.attr_stride_c, 2, H / 2, W / 2, "attribute V");
+      }
+    }
+  return n;
+}
+
 // Device planes (TMC2_INPUT_DEVICE): the allocations they were found in, with their devices.  A plane inside an allocation
 // already seen costs no driver call (a GOF held in one tensor is checked with one query per plane kind).
 struct DevRange { uintptr_t base; size_t size; int device; };
 
-static tmc2_status check_device_plane(const void* p, uint32_t rows, size_t pitch_bytes, size_t row_bytes, const std::vector<int>& devices,
-                                      std::vector<DevRange>& ranges, uint32_t f, const char* what, Err& err) {
-  const uintptr_t a = (uintptr_t)p;
-  const size_t extent = (size_t)(rows - 1) * pitch_bytes + row_bytes;
+static tmc2_status check_device_plane(const SrcPlane& sp, const std::vector<int>& devices, std::vector<DevRange>& ranges, uint32_t f,
+                                      Err& err) {
+  const uintptr_t a = (uintptr_t)sp.p;
+  const size_t extent = sp.extent();
+  const char* what = sp.name;
   for (const DevRange& r : ranges)
     if (a >= r.base && a - r.base < r.size) {
       if (extent > r.size - (a - r.base))
@@ -324,7 +365,7 @@ static tmc2_status check_device_plane(const void* p, uint32_t rows, size_t pitch
       return TMC2_OK;
     }
   cudaPointerAttributes at{};
-  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+  if (cudaPointerGetAttributes(&at, sp.p) != cudaSuccess) {
     cudaGetLastError();
     FAIL(TMC2_ERR_INVALID_ARG, "frame %u: %s plane is not CUDA device memory (TMC2_INPUT_DEVICE)", f, what);
   }
@@ -355,7 +396,6 @@ static tmc2_status validate_frame(const tmc2_gof* g, uint32_t f, const std::vect
                                   Err& err) {
   const tmc2_params& P = g->params;
   const tmc2_frame& fr = g->frames[f];
-  const bool p010 = (g->input_flags & TMC2_INPUT_P010) != 0;
   // codec.rs:318-320: geometry video must hold frames f*M .. f*M+M-1
   if ((uint64_t)g->geo_video_frames < (uint64_t)f * 2 + 2)
     FAIL(TMC2_ERR_SHORT_VIDEO, "geometry video has %u frames, frame %u needs %llu (codec.rs:318)", g->geo_video_frames, f,
@@ -363,16 +403,14 @@ static tmc2_status validate_frame(const tmc2_gof* g, uint32_t f, const std::vect
   if (P.attribute_count && (uint64_t)g->attr_video_frames < (uint64_t)f * 2 + 2)
     FAIL(TMC2_ERR_SHORT_VIDEO, "attribute video has %u frames, frame %u needs %llu (codec.rs:589,637)",
          g->attr_video_frames, f, (unsigned long long)f * 2 + 2);
-  if (!fr.occ || !fr.geo[0] || !fr.geo[1]) FAIL(TMC2_ERR_INVALID_ARG, "frame %u: NULL occupancy / geometry plane", f);
-  if (P.attribute_count && (!fr.attr_y[0] || !fr.attr_y[1] || !fr.attr_u[0] || !fr.attr_u[1] ||
-                            (!p010 && (!fr.attr_v[0] || !fr.attr_v[1]))))
-    FAIL(TMC2_ERR_INVALID_ARG, "frame %u: NULL attribute plane", f);
-  if (P.attribute_count && p010 && (fr.attr_v[0] || fr.attr_v[1]))
+  SrcPlane src[kMaxFramePlanes];
+  const uint32_t n_src = frame_planes(g, f, src);
+  for (uint32_t i = 0; i < n_src; ++i)
+    if (!src[i].p) FAIL(TMC2_ERR_INVALID_ARG, "frame %u: NULL %s plane", f, src[i].kind <= kGeo ? "occupancy / geometry" : "attribute");
+  if (P.attribute_count && (g->input_flags & TMC2_INPUT_P010) && (fr.attr_v[0] || fr.attr_v[1]))
     FAIL(TMC2_ERR_INVALID_ARG, "frame %u: attr_v must be NULL with TMC2_INPUT_P010 (attr_u is the interleaved UV plane)", f);
-  // P010: attr_u rows hold width/2 interleaved (U, V) pairs = width elements
-  if (fr.occ_stride < g->occ_width || fr.geo_stride < g->width ||
-      (P.attribute_count && (fr.attr_stride_y < g->width || fr.attr_stride_c < (p010 ? g->width : g->width / 2))))
-    FAIL(TMC2_ERR_INVALID_ARG, "frame %u: stride smaller than width", f);
+  for (uint32_t i = 0; i < n_src; ++i)
+    if (src[i].pitch < src[i].row_bytes) FAIL(TMC2_ERR_INVALID_ARG, "frame %u: stride smaller than width", f);
   if (fr.patch_count && !fr.patches) FAIL(TMC2_ERR_INVALID_ARG, "frame %u: NULL patch list", f);
   if (fr.patch_count > 65535) FAIL(TMC2_ERR_CAPACITY, "frame %u: more than 65535 patches", f);
   const int64_t res = P.occupancy_resolution;
@@ -407,23 +445,9 @@ static tmc2_status validate_frame(const tmc2_gof* g, uint32_t f, const std::vect
              (long long)x, (long long)y);
     }
   }
-  if (g->input_flags & TMC2_INPUT_DEVICE) {
-    if (check_device_plane(fr.occ, g->occ_height, fr.occ_stride, g->occ_width, devices, ranges, f, "occupancy", err)) return err.st;
-    for (int m = 0; m < 2; ++m)
-      if (check_device_plane(fr.geo[m], g->height, (size_t)fr.geo_stride * 2, (size_t)g->width * 2, devices, ranges, f, "geometry", err))
-        return err.st;
-    if (P.attribute_count) {
-      const uint32_t hc = g->height / 2;
-      for (int m = 0; m < 2; ++m) {
-        if (check_device_plane(fr.attr_y[m], g->height, (size_t)fr.attr_stride_y * 2, (size_t)g->width * 2, devices, ranges, f,
-                               "attribute Y", err)) return err.st;
-        if (check_device_plane(fr.attr_u[m], hc, (size_t)fr.attr_stride_c * 2, (size_t)(p010 ? g->width : g->width / 2) * 2, devices,
-                               ranges, f, p010 ? "attribute UV" : "attribute U", err)) return err.st;
-        if (!p010 && check_device_plane(fr.attr_v[m], hc, (size_t)fr.attr_stride_c * 2, (size_t)(g->width / 2) * 2, devices, ranges, f,
-                                        "attribute V", err)) return err.st;
-      }
-    }
-  }
+  if (g->input_flags & TMC2_INPUT_DEVICE)
+    for (uint32_t i = 0; i < n_src; ++i)
+      if (check_device_plane(src[i], devices, ranges, f, err)) return err.st;
   return TMC2_OK;
 }
 
@@ -435,7 +459,16 @@ enum : uint32_t {
   WANT_OCC_FULL = 2u,    // materialise tile.occupancy_map (K1)
 };
 
-struct StageTimes { float b2p = 0, count = 0, unpack = 0, geo = 0, col = 0, rgb = 0; };
+struct StageTimes { float b2p = 0, count = 0, unpack = 0, geo = 0; };
+
+// One plane kind in the batch layout (device_types.h): F frames x `maps` planes of h rows of `pitch` elements
+struct PlaneDesc {
+  uint32_t esz = 1, maps = 1, w = 0, h = 0, pitch = 0;
+  DevBuf buf;
+  uint64_t elems() const { return (uint64_t)h * pitch; }   // one plane
+  uint64_t bytes() const { return elems() * esz; }
+  uint8_t* at(uint32_t frame, uint32_t map) const { return buf.as<uint8_t>() + ((size_t)frame * maps + map) * bytes(); }
+};
 
 struct Batch {
   int device = 0;
@@ -445,11 +478,10 @@ struct Batch {
   std::vector<cudaEvent_t> ev_emit, ev_post;   // per group: emit done (main stream) / filter+clear done (aux)
   cudaEvent_t ev_tables_clean = nullptr;       // single-group launches: the clear pass runs on aux, off the critical path
   bool clear_pending = false;
-  bool two_pass = false;
 
   // description of the loaded GOF slice
   uint32_t W = 0, H = 0, occ_w = 0, occ_h = 0, F = 0, res = 16, prec = 4;
-  uint32_t geo_pitch = 0, attr_pitch_y = 0, attr_pitch_c = 0, occ_pitch = 0, Hc = 0;
+  PlaneDesc planes[kPlaneKinds];      // the plane arrays, by PlaneKind
   tmc2_params params{};
   uint32_t want = 0;
   uint64_t cap = 0;                   // points per frame slab
@@ -460,7 +492,7 @@ struct Batch {
   std::vector<SlotRec> h_slot_rec;
   std::vector<uint32_t> h_tile_frame, h_ftb;
 
-  DevBuf d_occ, d_geo, d_ay, d_au, d_av, d_meta, d_b2p, d_count, d_err, d_work, d_owned_count, d_slot_bt, d_slot_bbase, d_slot_nmin;
+  DevBuf d_meta, d_b2p, d_count, d_err, d_work, d_owned_count, d_slot_bt, d_slot_bbase, d_slot_nmin;
   DevBuf d_pos, d_rgb, d_yuv, d_part, d_pix, d_bt, d_occ_full, d_pos_pre, d_yuv_pre;
   DevBuf d_geotab, d_coltab, d_geokeys, d_colkeys, d_changed, d_blist,
       d_blist_count, d_slist, d_slist_count, d_geombits, d_colmbits, d_geotbits, d_coltbits;
@@ -474,10 +506,12 @@ struct Batch {
   DevBuf d_ply, d_ply_sums;           // tmc2gpu_frame_to_ply: body scratch, block sums + offsets + total
   size_t meta_patch_off = 0, meta_slot_off = 0, meta_tf_off = 0, meta_ftb_off = 0, meta_ingest_off = 0, meta_bytes = 0;
   uint32_t input_flags = 0;           // tmc2_gof.input_flags of the loaded GOF
-  uint32_t n_ingest = 0;              // device planes: entries of the ingest table (end of the metadata block)
   uint32_t ingest_launches = 0;       // ingest kernel launched by upload(), counted with the next launch()
 
-  cudaEvent_t ev[8] = {};             // stage boundaries: 0 start,1 after b2p,2 after unpack,3 geo,4 col,5 rgb
+  // stage-timing events of a timed launch: start, block-to-patch done, around the count + scan passes, unpack (emit and
+  // smoothing) done, launch done
+  enum { EV_START, EV_B2P, EV_COUNT0, EV_COUNT1, EV_UNPACK, EV_DONE, N_EV };
+  cudaEvent_t ev[N_EV] = {};
   cudaEvent_t ev_counts = nullptr, ev_inputs_free = nullptr;
   std::vector<cudaEvent_t> ev_frame;  // per-frame D2H completion
 
@@ -500,7 +534,8 @@ struct Batch {
   ~Batch() { destroy(); }
   void destroy() {
     cudaSetDevice(device);
-    for (DevBuf* b : {&d_occ, &d_geo, &d_ay, &d_au, &d_av, &d_meta, &d_b2p, &d_count, &d_err, &d_work,
+    for (PlaneDesc& pl : planes) pl.buf.release();
+    for (DevBuf* b : {&d_meta, &d_b2p, &d_count, &d_err, &d_work,
                       &d_owned_count, &d_slot_bt, &d_slot_bbase, &d_slot_nmin, &d_pos,
                       &d_rgb, &d_yuv, &d_part, &d_pix, &d_bt, &d_occ_full, &d_pos_pre, &d_yuv_pre, &d_geotab, &d_coltab,
                       &d_geokeys, &d_colkeys, &d_changed, &d_blist,
@@ -525,8 +560,8 @@ struct Batch {
     if (d2h_stream) cudaStreamDestroy(d2h_stream), d2h_stream = nullptr;
   }
 
-  tmc2_status init(int dev, bool two_pass_scan, Err& err) {
-    device = dev; two_pass = two_pass_scan;
+  tmc2_status init(int dev, Err& err) {
+    device = dev;
     CU(cudaSetDevice(device));
     CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&d2h_stream, cudaStreamNonBlocking));
@@ -554,15 +589,20 @@ struct Batch {
     bw = W / res; bh = H / res;
     want = want_flags;
     input_flags = g->input_flags;
-    Hc = H / 2;
-    geo_pitch = round_up(W, 64); attr_pitch_y = round_up(W, 64); attr_pitch_c = round_up(std::max(W / 2, 1u), 64);
-    occ_pitch = round_up(occ_w, 16);
+    auto describe = [&](uint32_t kind, uint32_t esz, uint32_t maps, uint32_t w, uint32_t h, uint32_t pitch_align) {
+      PlaneDesc& pl = planes[kind];
+      pl.esz = esz; pl.maps = maps; pl.w = w; pl.h = h; pl.pitch = round_up(w, pitch_align);
+    };
+    describe(kOcc, 1, 1, occ_w, occ_h, 16);
+    describe(kGeo, 2, 2, W, H, 64);
+    describe(kAttrY, 2, 2, W, H, 64);
+    describe(kAttrU, 2, 2, std::max(W / 2, 1u), std::max(H / 2, 1u), 64);
+    describe(kAttrV, 2, 2, std::max(W / 2, 1u), std::max(H / 2, 1u), 64);
     cap = round_up64(2ull * W * H, 16);   // slabs stay 16-byte aligned for both output streams
     smoothing_geo = params.geometry_smoothing != 0;
     smoothing_col = params.color_smoothing != 0 && params.attribute_count != 0;
 
     h_patches.clear(); h_slot_rec.clear(); h_tile_frame.clear(); h_ftb.assign(1, 0);
-    uint64_t total_points_bound = 0;
     for (uint32_t k = 0; k < count; ++k) {
       const tmc2_frame& fr = g->frames[first + k];
       for (uint32_t i = 0; i < fr.patch_count; ++i) {
@@ -597,7 +637,6 @@ struct Batch {
             if (!d.aligned) { r.ax = r.ay = r.rx = r.ry = 0; }   // reference-literal rotated patch: generic device path
             h_slot_rec.push_back(r);
           }
-        total_points_bound += ns * res * res * 2;
       }
       // pad the frame's slot list to whole tiles: a tile never straddles two frames (one scan domain per frame)
       while (h_slot_rec.size() % kWarpsPerTile) { SlotRec r{}; r.pid = kNoPatch; h_slot_rec.push_back(r); }
@@ -607,25 +646,17 @@ struct Batch {
     }
     n_slots = (uint32_t)h_slot_rec.size();
     n_tiles = n_slots / kWarpsPerTile;
-    (void)total_points_bound;
 
     // device buffers
     const bool attr = params.attribute_count != 0;
-    CU(d_occ.ensure((size_t)F * occ_h * occ_pitch));
-    CU(d_geo.ensure((size_t)F * 2 * H * geo_pitch * 2));
-    if (attr) {
-      CU(d_ay.ensure((size_t)F * 2 * H * attr_pitch_y * 2));
-      CU(d_au.ensure((size_t)F * 2 * std::max(Hc, 1u) * attr_pitch_c * 2));
-      CU(d_av.ensure((size_t)F * 2 * std::max(Hc, 1u) * attr_pitch_c * 2));
-    }
+    for (uint32_t kind = 0; kind < n_kinds(); ++kind) CU(planes[kind].buf.ensure((size_t)F * planes[kind].maps * planes[kind].bytes()));
+    pair_planes(g, first);
     meta_patch_off = 0;
     meta_slot_off = round_up64(h_patches.size() * sizeof(DevPatch), 256);
     meta_tf_off = meta_slot_off + round_up64((uint64_t)n_slots * sizeof(SlotRec), 256);
     meta_ftb_off = meta_tf_off + round_up64((uint64_t)n_tiles * 4, 256);
     meta_ingest_off = meta_ftb_off + round_up64((uint64_t)(F + 1) * 4, 256);
-    // one table entry per (frame, kind, map): occupancy, 2 geometry, 2 luma, 2 UV (P010) or 2 U + 2 V
-    n_ingest = (input_flags & TMC2_INPUT_DEVICE) ? F * (3 + (attr ? ((input_flags & TMC2_INPUT_P010) ? 4 : 6) : 0)) : 0;
-    meta_bytes = meta_ingest_off + (size_t)n_ingest * sizeof(IngestPlane);
+    meta_bytes = meta_ingest_off + ((input_flags & TMC2_INPUT_DEVICE) ? segs.size() * sizeof(IngestPlane) : 0);
     CU(d_meta.ensure(meta_bytes));
     CU(h_meta.ensure(meta_bytes));
     CU(d_b2p.ensure(std::max<size_t>((size_t)F * bw * bh * 4, 4)));
@@ -728,61 +759,51 @@ struct Batch {
     return make_tile_maps(err);
   }
 
+  // ---- planes in: a caller plane and the batch plane it lands in ---------------------------------------------------
+  struct Seg {
+    SrcPlane src;
+    uint8_t* dst; size_t dpb, plane_dev;   // batch plane: pointer, pitch in bytes, bytes of the plane on the device
+    bool staged; size_t stage_off;         // host planes: repacked into pinned staging at stage_off
+  };
+  std::vector<Seg> segs;                   // every plane of the loaded frames (pair_planes)
+  uint32_t n_kinds() const { return params.attribute_count ? kPlaneKinds : kAttrY; }
+
+  // Pairs every caller plane of frames first .. first+F-1 with its batch plane: kind by kind, then frame, then map, which is
+  // the order of the batch layout (neighbouring planes can merge into one copy, and the staging groups follow it).
+  void pair_planes(const tmc2_gof* g, uint32_t first) {
+    segs.clear();
+    for (uint32_t kind = 0; kind < n_kinds(); ++kind)
+      for (uint32_t k = 0; k < F; ++k) {
+        SrcPlane src[kMaxFramePlanes];
+        const uint32_t n = frame_planes(g, first + k, src);
+        const PlaneDesc& pl = planes[kind];
+        for (uint32_t i = 0; i < n; ++i)
+          if (src[i].kind == kind) segs.push_back({src[i], pl.at(k, src[i].map), (size_t)pl.pitch * pl.esz, pl.bytes(), false, 0});
+      }
+  }
+
   // ---- H2D: planes (through pinned staging unless the caller's memory is already pinned) + metadata -------------
   // One row-pitched copy per (frame, map), merged when neighbouring planes are contiguous on both sides.  Whether a plane is
   // DMA'd in place or staged is decided ONCE per plane, on its full extent, and the staging area is sized from exactly
   // those decisions.
-  struct Seg {
-    const uint8_t* src; size_t spitch; uint8_t* dst; uint32_t rows;
-    size_t row_bytes, dpb, plane_dev;      // bytes per row, device pitch in bytes, bytes of the plane on the device
-    bool staged; size_t stage_off;
-    int kind;                              // runs are only merged inside one device allocation (= one plane kind)
-  };
-  void plan_plane_set(const tmc2_gof* g, uint32_t first, int kind, const std::vector<std::pair<const uint8_t*, size_t>>& reg,
-                      std::vector<Seg>& segs, size_t& stage_bytes) const {
-    // kind: 0 occ, 1 geo, 2 attr_y, 3 attr_u, 4 attr_v
-    const int maps = kind == 0 ? 1 : 2;
-    const uint32_t esz = kind == 0 ? 1 : 2;
-    const uint32_t w = kind == 0 ? occ_w : (kind >= 3 ? W / 2 : W);
-    const uint32_t h = kind == 0 ? occ_h : (kind >= 3 ? Hc : H);
-    const uint32_t dpitch = kind == 0 ? occ_pitch : kind == 1 ? geo_pitch : kind == 2 ? attr_pitch_y : attr_pitch_c;
-    uint8_t* dbase = kind == 0 ? d_occ.as<uint8_t>() : kind == 1 ? d_geo.as<uint8_t>() : kind == 2 ? d_ay.as<uint8_t>()
-                   : kind == 3 ? d_au.as<uint8_t>() : d_av.as<uint8_t>();
-    if (w == 0 || h == 0) return;
-    const size_t plane_dev = (size_t)h * dpitch * esz;
-    for (uint32_t k = 0; k < F; ++k) {
-      const tmc2_frame& fr = g->frames[first + k];
-      for (int m = 0; m < maps; ++m) {
-        const void* src = kind == 0 ? (const void*)fr.occ : kind == 1 ? (const void*)fr.geo[m]
-                        : kind == 2 ? (const void*)fr.attr_y[m] : kind == 3 ? (const void*)fr.attr_u[m] : (const void*)fr.attr_v[m];
-        const uint32_t sstride = kind == 0 ? fr.occ_stride : kind == 1 ? fr.geo_stride : kind == 2 ? fr.attr_stride_y : fr.attr_stride_c;
-        Seg s{(const uint8_t*)src, (size_t)sstride * esz, dbase + ((size_t)k * maps + m) * plane_dev, h,
-              (size_t)w * esz, (size_t)dpitch * esz, plane_dev, false, 0, kind};
-        const size_t src_bytes = (size_t)(s.rows - 1) * s.spitch + s.row_bytes;
-        s.staged = !is_pinned(reg, s.src, src_bytes);
-        if (s.staged) { s.stage_off = stage_bytes; stage_bytes += plane_dev; }
-        segs.push_back(s);
-      }
-    }
-  }
-
   // dev_ranges: allocations of the GOF's device planes (validate_frame), for TMC2_INPUT_DEVICE
-  tmc2_status upload(const tmc2_gof* g, uint32_t first, const std::vector<DevRange>& dev_ranges, Err& err, bool use_pool = true) {
+  tmc2_status upload(const std::vector<DevRange>& dev_ranges, Err& err, bool use_pool = true) {
     CU(cudaSetDevice(device));
-    if (input_flags & TMC2_INPUT_DEVICE) return upload_device(g, first, dev_ranges, err);
-    const bool attr = params.attribute_count != 0;
-    std::vector<Seg> segs;
+    if (input_flags & TMC2_INPUT_DEVICE) return upload_device(dev_ranges, err);
     size_t stage_bytes = 0;
     {
       const auto reg = pinned_snapshot();
-      for (int kind = 0; kind < (attr ? 5 : 2); ++kind) plan_plane_set(g, first, kind, reg, segs, stage_bytes);
+      for (Seg& s : segs) {
+        s.staged = !is_pinned(reg, s.src.p, s.src.extent());
+        if (s.staged) { s.stage_off = stage_bytes; stage_bytes += s.plane_dev; }
+      }
     }
     // the previous GOF of this batch must have finished its H2D copies before its staging area (planes and metadata) is
     // written again
     CU(cudaEventSynchronize(ev_inputs_free));
     if (stage_bytes) CU(h_in.ensure(stage_bytes));
     // current run of planes that are contiguous on both sides -> one cudaMemcpyAsync
-    const uint8_t* run_src = nullptr; uint8_t* run_dst = nullptr; size_t run_bytes = 0; int run_kind = -1;
+    const uint8_t* run_src = nullptr; uint8_t* run_dst = nullptr; size_t run_bytes = 0; uint32_t run_kind = 0;
     auto flush = [&]() -> cudaError_t {
       cudaError_t e = cudaSuccess;
       if (run_bytes) e = cudaMemcpyAsync(run_dst, run_src, run_bytes, cudaMemcpyHostToDevice, stream);
@@ -790,19 +811,20 @@ struct Batch {
       return e;
     };
     auto enqueue = [&](const Seg& s) -> tmc2_status {
-      const uint8_t* src = s.staged ? h_in.as<uint8_t>() + s.stage_off : s.src;
-      const size_t spitch = s.staged ? s.dpb : s.spitch;
+      const uint8_t* src = s.staged ? h_in.as<uint8_t>() + s.stage_off : s.src.p;
+      const size_t spitch = s.staged ? s.dpb : s.src.pitch;
       // in-place planes: the last row of a plane may be shorter than the pitch in the SOURCE allocation -- never read past it
-      if (spitch == s.dpb && (s.staged || s.row_bytes == s.dpb)) {
-        if (run_bytes && s.kind == run_kind && src == run_src + run_bytes && s.dst == run_dst + run_bytes) {
+      // (runs are only merged inside one device allocation = one plane kind)
+      if (spitch == s.dpb && (s.staged || s.src.row_bytes == s.dpb)) {
+        if (run_bytes && s.src.kind == run_kind && src == run_src + run_bytes && s.dst == run_dst + run_bytes) {
           run_bytes += s.plane_dev;
         } else {
           CU(flush());
-          run_src = src; run_dst = s.dst; run_bytes = s.plane_dev; run_kind = s.kind;
+          run_src = src; run_dst = s.dst; run_bytes = s.plane_dev; run_kind = s.src.kind;
         }
       } else {
         CU(flush());
-        CU(cudaMemcpy2DAsync(s.dst, s.dpb, src, spitch, s.row_bytes, s.rows, cudaMemcpyHostToDevice, stream));
+        CU(cudaMemcpy2DAsync(s.dst, s.dpb, src, spitch, s.src.row_bytes, s.src.rows, cudaMemcpyHostToDevice, stream));
       }
       return TMC2_OK;
     };
@@ -819,15 +841,17 @@ struct Batch {
         for (size_t k = i; k < j; ++k) {
           if (!segs[k].staged) continue;
           const uint32_t rows_per = std::max<uint32_t>(1, (uint32_t)((1u << 20) / std::max<size_t>(segs[k].dpb, 1)));   // ~1 MB pieces
-          for (uint32_t r = 0; r < segs[k].rows; r += rows_per) items.push_back({&segs[k], r, std::min(segs[k].rows, r + rows_per)});
+          const uint32_t rows = segs[k].src.rows;
+          for (uint32_t r = 0; r < rows; r += rows_per) items.push_back({&segs[k], r, std::min(rows, r + rows_per)});
         }
         uint8_t* base = h_in.as<uint8_t>();
         auto stage_item = [&](size_t n) {
           const Item& it = items[n];
           const Seg& sg = *it.s;
+          const SrcPlane& sp = sg.src;
           uint8_t* st = base + sg.stage_off;
-          if (sg.spitch == sg.dpb && sg.row_bytes == sg.dpb) memcpy(st + (size_t)it.r0 * sg.dpb, sg.src + (size_t)it.r0 * sg.spitch, (size_t)(it.r1 - it.r0) * sg.dpb);
-          else for (uint32_t r = it.r0; r < it.r1; ++r) memcpy(st + (size_t)r * sg.dpb, sg.src + (size_t)r * sg.spitch, sg.row_bytes);
+          if (sp.pitch == sg.dpb && sp.row_bytes == sg.dpb) memcpy(st + (size_t)it.r0 * sg.dpb, sp.p + (size_t)it.r0 * sp.pitch, (size_t)(it.r1 - it.r0) * sg.dpb);
+          else for (uint32_t r = it.r0; r < it.r1; ++r) memcpy(st + (size_t)r * sg.dpb, sp.p + (size_t)r * sp.pitch, sp.row_bytes);
         };
         if (use_pool) StagePool::get().run(items.size(), stage_item);
         else for (size_t n = 0; n < items.size(); ++n) stage_item(n);     // already on a pool thread (one per device piece)
@@ -854,7 +878,7 @@ struct Batch {
 
   // TMC2_INPUT_DEVICE: no staging and no H2D of planes.  The planes' table goes with the metadata, and one kernel gathers
   // every plane into the batch layout (the same layout the host path produces, so everything downstream is unchanged).
-  tmc2_status upload_device(const tmc2_gof* g, uint32_t first, const std::vector<DevRange>& dev_ranges, Err& err) {
+  tmc2_status upload_device(const std::vector<DevRange>& dev_ranges, Err& err) {
     for (const DevRange& r : dev_ranges) {
       if (r.device == device) continue;
       int can = 0;
@@ -866,42 +890,25 @@ struct Batch {
     }
     // the previous GOF of this batch must have been read (ingest done, metadata copied) before its table is written again
     CU(cudaEventSynchronize(ev_inputs_free));
-    const bool attr = params.attribute_count != 0, p010 = (input_flags & TMC2_INPUT_P010) != 0;
+    const bool p010 = (input_flags & TMC2_INPUT_P010) != 0;
     IngestPlane* tab = reinterpret_cast<IngestPlane*>(h_meta.as<uint8_t>() + meta_ingest_off);
-    uint32_t n = 0, max_rows = 0, max_row_bytes = 0;
-    auto add = [&](const void* src, size_t spitch, uint32_t rows, uint32_t row_bytes, uint8_t* dst, uint8_t* dst2, uint32_t dpitch,
-                   uint32_t op) {
-      IngestPlane& e = tab[n++];
-      e.src = static_cast<const uint8_t*>(src); e.dst = dst; e.dst2 = dst2;
-      e.spitch = (uint32_t)spitch; e.dpitch = dpitch; e.rows = rows; e.row_bytes = row_bytes;
-      e.op = op | (((uintptr_t)src % 16 == 0 && spitch % 16 == 0) ? (uint32_t)kIngestVec : 0u);
+    uint32_t max_rows = 0, max_row_bytes = 0;
+    for (size_t i = 0; i < segs.size(); ++i) {
+      const Seg& s = segs[i];
+      const SrcPlane& sp = s.src;
+      const bool uv = p010 && sp.kind == kAttrU;   // interleaved UV: V lands at the same offset of the V plane array
+      const uint32_t op = sp.kind == kOcc ? kIngestCopy8 : uv ? kIngestUv16 : p010 ? kIngestShr16 : kIngestCopy16;
+      IngestPlane& e = tab[i];
+      e.src = sp.p; e.dst = s.dst;
+      e.dst2 = uv ? planes[kAttrV].buf.as<uint8_t>() + (s.dst - planes[kAttrU].buf.as<uint8_t>()) : nullptr;
+      e.spitch = (uint32_t)sp.pitch; e.dpitch = (uint32_t)s.dpb; e.rows = sp.rows; e.row_bytes = (uint32_t)sp.row_bytes;
+      e.op = op | (((uintptr_t)sp.p % 16 == 0 && sp.pitch % 16 == 0) ? (uint32_t)kIngestVec : 0u);
       e._pad = 0;
-      max_rows = std::max(max_rows, rows); max_row_bytes = std::max(max_row_bytes, row_bytes);
-    };
-    const uint32_t op16 = p010 ? kIngestShr16 : kIngestCopy16;
-    const size_t occ_plane = (size_t)occ_h * occ_pitch, geo_plane = (size_t)H * geo_pitch * 2, y_plane = (size_t)H * attr_pitch_y * 2;
-    const size_t c_plane = (size_t)std::max(Hc, 1u) * attr_pitch_c * 2;
-    for (uint32_t k = 0; k < F; ++k) {
-      const tmc2_frame& fr = g->frames[first + k];
-      add(fr.occ, fr.occ_stride, occ_h, occ_w, d_occ.as<uint8_t>() + k * occ_plane, nullptr, occ_pitch, kIngestCopy8);
-      for (uint32_t m = 0; m < 2; ++m) {
-        const size_t km = (size_t)k * 2 + m;
-        add(fr.geo[m], (size_t)fr.geo_stride * 2, H, W * 2, d_geo.as<uint8_t>() + km * geo_plane, nullptr, geo_pitch * 2, op16);
-        if (!attr) continue;
-        add(fr.attr_y[m], (size_t)fr.attr_stride_y * 2, H, W * 2, d_ay.as<uint8_t>() + km * y_plane, nullptr, attr_pitch_y * 2, op16);
-        if (p010) {
-          add(fr.attr_u[m], (size_t)fr.attr_stride_c * 2, Hc, W * 2, d_au.as<uint8_t>() + km * c_plane, d_av.as<uint8_t>() + km * c_plane,
-              attr_pitch_c * 2, kIngestUv16);
-        } else {
-          add(fr.attr_u[m], (size_t)fr.attr_stride_c * 2, Hc, (W / 2) * 2, d_au.as<uint8_t>() + km * c_plane, nullptr, attr_pitch_c * 2, op16);
-          add(fr.attr_v[m], (size_t)fr.attr_stride_c * 2, Hc, (W / 2) * 2, d_av.as<uint8_t>() + km * c_plane, nullptr, attr_pitch_c * 2, op16);
-        }
-      }
+      max_rows = std::max(max_rows, e.rows); max_row_bytes = std::max(max_row_bytes, e.row_bytes);
     }
-    if (n != n_ingest) FAIL(TMC2_ERR_INTERNAL, "ingest table: %u entries, %u expected", n, n_ingest);
     if (send_meta(err)) return err.st;
-    KL(launch_ingest_planes(reinterpret_cast<const IngestPlane*>(d_meta.as<uint8_t>() + meta_ingest_off), n, max_rows, max_row_bytes,
-                            stream));
+    KL(launch_ingest_planes(reinterpret_cast<const IngestPlane*>(d_meta.as<uint8_t>() + meta_ingest_off), (uint32_t)segs.size(), max_rows,
+                            max_row_bytes, stream));
     ingest_launches = 1;
     CU(cudaEventRecord(ev_inputs_free, stream));
     return TMC2_OK;
@@ -912,41 +919,32 @@ struct Batch {
   tmc2_status make_tile_maps(Err& err) {
     memset(&tile_maps, 0, sizeof tile_maps);
     if (F == 0 || res != 16) return TMC2_OK;                           // no block-aligned slots: the maps are never used
-    const uint64_t gms = (uint64_t)H * geo_pitch * 2, yms = (uint64_t)H * attr_pitch_y * 2, cms = (uint64_t)std::max(Hc, 1u) * attr_pitch_c * 2;
-    bool ok = true;
-    {
-      const uint64_t dims[4] = {W, H, 2, F}, st[3] = {(uint64_t)geo_pitch * 2, gms, 2 * gms};
-      const uint32_t box[4] = {16, 16, 2, 1};
-      ok &= encode_map(tile_maps.geo, d_geo.p, 2, 4, dims, st, box);
-    }
-    if (params.attribute_count) {
-      const uint64_t dims[4] = {W, H, 2, F}, st[3] = {(uint64_t)attr_pitch_y * 2, yms, 2 * yms};
-      const uint32_t box[4] = {16, 16, 2, 1};
-      ok &= encode_map(tile_maps.attr_y, d_ay.p, 2, 4, dims, st, box);
-      const uint64_t cd[4] = {std::max(W / 2, 1u), std::max(Hc, 1u), 2, F}, cs[3] = {(uint64_t)attr_pitch_c * 2, cms, 2 * cms};
-      const uint32_t cbox[4] = {8, 8, 2, 1};
-      ok &= encode_map(tile_maps.attr_u, d_au.p, 2, 4, cd, cs, cbox);
-      ok &= encode_map(tile_maps.attr_v, d_av.p, 2, 4, cd, cs, cbox);
-    }
-    {
-      const uint64_t dims[3] = {occ_w, occ_h, F}, st[2] = {(uint64_t)occ_pitch, (uint64_t)occ_h * occ_pitch};
-      const uint32_t box[3] = {32, 8, 1};
-      ok &= encode_map(tile_maps.occ, d_occ.p, 1, 3, dims, st, box);
-    }
+    // (x, y, map, frame); a kind with one map (occupancy) is (x, y, frame)
+    auto map = [&](unsigned long long* out, uint32_t kind, uint32_t bx, uint32_t by) {
+      const PlaneDesc& pl = planes[kind];
+      const bool one = pl.maps == 1;
+      const uint64_t dims[4] = {pl.w, pl.h, one ? F : pl.maps, F}, st[3] = {(uint64_t)pl.pitch * pl.esz, pl.bytes(), pl.maps * pl.bytes()};
+      const uint32_t box[4] = {bx, by, one ? 1u : pl.maps, 1};
+      return encode_map(out, pl.buf.p, pl.esz, one ? 3 : 4, dims, st, box);
+    };
+    bool ok = map(tile_maps.geo, kGeo, 16, 16) && map(tile_maps.occ, kOcc, 32, 8);
+    if (params.attribute_count)
+      ok = ok && map(tile_maps.attr_y, kAttrY, 16, 16) && map(tile_maps.attr_u, kAttrU, 8, 8) && map(tile_maps.attr_v, kAttrV, 8, 8);
     if (!ok) FAIL(TMC2_ERR_CUDA, "cuTensorMapEncodeTiled failed (TMA descriptors of the plane arrays)");
     return TMC2_OK;
   }
 
   UnpackArgs make_args() const {
     UnpackArgs a{};
-    a.in.occ = d_occ.as<uint8_t>(); a.in.geo = d_geo.as<uint16_t>();
-    a.in.attr_y = d_ay.as<uint16_t>(); a.in.attr_u = d_au.as<uint16_t>(); a.in.attr_v = d_av.as<uint16_t>();
-    a.in.occ_pitch = occ_pitch; a.in.occ_w = occ_w; a.in.occ_h = occ_h;
-    a.in.geo_pitch = geo_pitch; a.in.attr_pitch_y = attr_pitch_y; a.in.attr_pitch_c = attr_pitch_c;
-    a.in.occ_frame_stride = (uint64_t)occ_h * occ_pitch;
-    a.in.geo_map_stride = (uint64_t)H * geo_pitch;
-    a.in.attr_y_map_stride = (uint64_t)H * attr_pitch_y;
-    a.in.attr_c_map_stride = (uint64_t)std::max(Hc, 1u) * attr_pitch_c;
+    const PlaneDesc &occ = planes[kOcc], &geo = planes[kGeo], &y = planes[kAttrY], &u = planes[kAttrU];
+    a.in.occ = occ.buf.as<uint8_t>(); a.in.geo = geo.buf.as<uint16_t>();
+    a.in.attr_y = y.buf.as<uint16_t>(); a.in.attr_u = u.buf.as<uint16_t>(); a.in.attr_v = planes[kAttrV].buf.as<uint16_t>();
+    a.in.occ_pitch = occ.pitch; a.in.occ_w = occ_w; a.in.occ_h = occ_h;
+    a.in.geo_pitch = geo.pitch; a.in.attr_pitch_y = y.pitch; a.in.attr_pitch_c = u.pitch;
+    a.in.occ_frame_stride = occ.elems();
+    a.in.geo_map_stride = geo.elems();
+    a.in.attr_y_map_stride = y.elems();
+    a.in.attr_c_map_stride = u.elems();
     a.W = W; a.H = H; a.res = res; a.prec = prec;
     a.prec_shift = -1;
     for (int s = 0; s < 16; ++s) if ((1u << s) == prec) a.prec_shift = s;
@@ -1017,8 +1015,11 @@ struct Batch {
 
   uint64_t algorithmic_bytes_core(uint64_t total_points) const {
     // SURVEY.md 8(d): occ + geometry Y (2 maps) + attribute YUV 4:2:0 (2 maps) + per-point output streams
-    uint64_t b = (uint64_t)F * ((uint64_t)occ_w * occ_h + 2ull * W * H * 2);
-    if (params.attribute_count) b += (uint64_t)F * 2ull * ((uint64_t)W * H + 2ull * (W / 2) * (H / 2)) * 2;
+    uint64_t b = 0;
+    for (uint32_t kind = 0; kind < n_kinds(); ++kind) {
+      const PlaneDesc& pl = planes[kind];
+      b += (uint64_t)F * pl.maps * pl.w * pl.h * pl.esz;        // samples the reference reads, without the pitch padding
+    }
     uint64_t per_point = 6;
     const bool dbg = (want & WANT_DEBUG) != 0;
     if (params.attribute_count) per_point += 3;
@@ -1032,12 +1033,12 @@ struct Batch {
     CU(cudaSetDevice(device));
     kernel_launch_count_reset();
     UnpackArgs a = make_args();
-    if (timed) CU(cudaEventRecord(ev[0], s));
+    if (timed) CU(cudaEventRecord(ev[EV_START], s));
     CU(cudaMemsetAsync(d_b2p.p, 0, std::max<size_t>((size_t)F * bw * bh * 4, 4), s));
     CU(cudaMemsetAsync(d_count.p, 0, std::max<size_t>((size_t)F * 4, 4), s));
     KL(launch_block_to_patch(a, n_slots, s));
     KL(launch_compact_owned(a, s));
-    if (timed) CU(cudaEventRecord(ev[1], s));
+    if (timed) CU(cudaEventRecord(ev[EV_B2P], s));
     const bool smooth = smoothing_geo || smoothing_col;
     const bool dbg = (want & WANT_DEBUG) != 0;
     CU(cudaMemsetAsync(d_changed.p, 0, std::max<size_t>((size_t)F * 16, 16), s));
@@ -1046,10 +1047,10 @@ struct Batch {
       CU(cudaMemsetAsync(d_slist_count.p, 0, std::max<size_t>((size_t)F * 4, 4), s));
     }
     // unpack = count (points per owned slot) -> slot scan (run starts per frame, frame totals) -> emit
-    if (timed) CU(cudaEventRecord(ev[6], s));
+    if (timed) CU(cudaEventRecord(ev[EV_COUNT0], s));
     KL(launch_count(a, 0, n_tiles, s));
     KL(launch_slot_scan(a, s));
-    if (timed) CU(cudaEventRecord(ev[7], s));
+    if (timed) CU(cudaEventRecord(ev[EV_COUNT1], s));
     if (!smooth) {
       while (ev_grp.size() < 2) { cudaEvent_t e; CU(cudaEventCreate(&e)); ev_grp.push_back(e); }
       n_groups = 1;
@@ -1112,13 +1113,13 @@ struct Batch {
       if (n_groups >= 2)
         for (uint32_t gi = n_groups - 2; gi < n_groups; ++gi) CU(cudaStreamWaitEvent(s, ev_post[gi], 0));
     }
-    if (timed) CU(cudaEventRecord(ev[2], s));
+    if (timed) CU(cudaEventRecord(ev[EV_UNPACK], s));
     if (want & WANT_OCC_FULL) KL(launch_upsample(a, d_occ_full.as<uint8_t>(), s));
     if (dbg && !smooth) {
       CU(cudaMemcpyAsync(d_pos_pre.p, d_pos.p, (size_t)F * cap * 6, cudaMemcpyDeviceToDevice, s));
       if (a.out.yuv) CU(cudaMemcpyAsync(d_yuv_pre.p, d_yuv.p, (size_t)F * cap * 6, cudaMemcpyDeviceToDevice, s));
     }
-    if (timed) CU(cudaEventRecord(ev[3], s)); if (timed) CU(cudaEventRecord(ev[4], s)); if (timed) CU(cudaEventRecord(ev[5], s));
+    if (timed) CU(cudaEventRecord(ev[EV_DONE], s));
     launches = (uint32_t)kernel_launch_count_reset() + ingest_launches;
     ingest_launches = 0;
     counts_ready = false; outputs_enqueued = false; counts_enqueued = false;
@@ -1211,11 +1212,11 @@ struct Batch {
 
   tmc2_status stage_times(StageTimes& t, Err& err) {
     CU(cudaSetDevice(device));
-    CU(cudaEventSynchronize(ev[5]));
-    CU(cudaEventElapsedTime(&t.b2p, ev[0], ev[1]));
+    CU(cudaEventSynchronize(ev[EV_DONE]));
+    CU(cudaEventElapsedTime(&t.b2p, ev[EV_START], ev[EV_B2P]));
     float whole = 0;
-    CU(cudaEventElapsedTime(&whole, ev[1], ev[2]));
-    CU(cudaEventElapsedTime(&t.count, ev[6], ev[7]));
+    CU(cudaEventElapsedTime(&whole, ev[EV_B2P], ev[EV_UNPACK]));
+    CU(cudaEventElapsedTime(&t.count, ev[EV_COUNT0], ev[EV_COUNT1]));
     t.unpack = 0;
     for (uint32_t gi = 0; gi < n_groups; ++gi) {
       float ms = 0;
@@ -1223,7 +1224,6 @@ struct Batch {
       t.unpack += ms;
     }
     t.geo = std::max(0.f, whole - t.unpack - t.count);   // filter + clear launches of all groups (both smoothing stages)
-    t.col = 0; t.rgb = 0;   // colour smoothing runs inside the same filter launch; RGB conversion is fused into the emit
     return TMC2_OK;
   }
 };
@@ -1250,7 +1250,6 @@ struct tmc2gpu_ctx {
   Err err;
   std::string last_error;
   Batch* last_batch = nullptr;                               // for launch info / stage times
-  bool two_pass = false;
   bool device_output = false;                                // TMC2_CTX_DEVICE_OUTPUT: frames stay in HBM
 
   tmc2_status fail() { last_error = err.msg; return err.st; }
@@ -1294,18 +1293,17 @@ tmc2_status tmc2gpu_create(const int* device_ids, int device_count, const tmc2_l
   if (limits) ctx->limits = *limits;
   if (ctx->limits.gofs_in_flight == 0) ctx->limits.gofs_in_flight = 2;
   if (ctx->limits.gofs_in_flight > 8) ctx->limits.gofs_in_flight = 8;
-  ctx->two_pass = (ctx->limits.flags & TMC2_CTX_TWO_PASS_SCAN) != 0;
   ctx->device_output = (ctx->limits.flags & TMC2_CTX_DEVICE_OUTPUT) != 0;
   ctx->slots.resize(ctx->devices.size());
   for (size_t d = 0; d < ctx->devices.size(); ++d) {
     for (uint32_t k = 0; k < ctx->limits.gofs_in_flight; ++k) {
       std::unique_ptr<Batch> b(new Batch());
-      if (b->init(ctx->devices[d], ctx->two_pass, ctx->err)) return ctx->err.st;
+      if (b->init(ctx->devices[d], ctx->err)) return ctx->err.st;
       ctx->slots[d].push_back(std::move(b));
     }
   }
   ctx->stage_batch.reset(new Batch());
-  if (ctx->stage_batch->init(ctx->devices[0], ctx->two_pass, ctx->err)) return ctx->err.st;
+  if (ctx->stage_batch->init(ctx->devices[0], ctx->err)) return ctx->err.st;
   *out_ctx = ctx.release();
   return TMC2_OK;
 }
@@ -1321,10 +1319,7 @@ const char* tmc2gpu_last_error(const tmc2gpu_ctx* ctx) { return ctx ? ctx->last_
 void* tmc2gpu_alloc_pinned(size_t bytes) {
   void* p = nullptr;
   if (bytes == 0) return nullptr;
-  // TMC2_PINNED_WC=1: write-combined pages (the host only ever writes decoded samples into these planes; the DMA engine
-  // reads them without snooping the CPU caches) -- an experiment knob, measured in profiles/
-  static const bool wc = [] { const char* e = getenv("TMC2_PINNED_WC"); return e && atoi(e) != 0; }();
-  if (cudaHostAlloc(&p, bytes, cudaHostAllocPortable | (wc ? cudaHostAllocWriteCombined : 0)) != cudaSuccess) { cudaGetLastError(); return nullptr; }
+  if (cudaHostAlloc(&p, bytes, cudaHostAllocPortable) != cudaSuccess) { cudaGetLastError(); return nullptr; }
   std::lock_guard<std::mutex> lk(g_pin_mu);
   g_pinned.emplace_back((const uint8_t*)p, bytes);
   return p;
@@ -1358,41 +1353,26 @@ tmc2_status tmc2gpu_submit_gof(tmc2gpu_ctx* ctx, const tmc2_gof* gof) {
     if (validate_frame(gof, f, ctx->devices, dev_ranges, err)) return ctx->fail();
   if (gof->frame_count == 0) return TMC2_OK;
 
-  // Frame-wise sharding: contiguous slices of the GOF, one per device; no collective (SURVEY.md 8e).  A device's slice can
-  // be cut further into chunks of TMC2_CHUNK_FRAMES frames, each an independent batch on its own stream (lower latency to
-  // the first frame); measured on B200 it does not raise throughput once several GOFs are in flight, so the default is
-  // one batch per device slice.
+  // Frame-wise sharding: contiguous slices of the GOF, one batch per device; no collective (SURVEY.md 8e).  Cutting a slice
+  // into smaller batches lowers the latency to the first frame but, measured on a B200, does not raise throughput once
+  // several GOFs are in flight.
   const uint32_t D = (uint32_t)ctx->devices.size();
   const uint32_t F = gof->frame_count;
-  static const uint32_t chunk_frames = [] { const char* e = getenv("TMC2_CHUNK_FRAMES"); return e ? (uint32_t)atoi(e) : 0u; }();
   struct Piece { uint32_t d, lo, hi; Batch* b; };
   std::vector<Piece> pieces;
   for (uint32_t d = 0; d < D; ++d) {
     const uint32_t lo = (uint32_t)((uint64_t)F * d / D), hi = (uint32_t)((uint64_t)F * (d + 1) / D);
-    const uint32_t step = chunk_frames ? chunk_frames : std::max(hi - lo, 1u);
-    for (uint32_t c = lo; c < hi; c += step) pieces.push_back({d, c, std::min(hi, c + step), nullptr});
+    if (lo < hi) pieces.push_back({d, lo, hi, nullptr});
   }
-  // every piece needs a free batch of its device; batches are created on demand, up to gofs_in_flight GOFs of this shape
-  for (uint32_t d = 0; d < D; ++d) {
-    uint32_t need = 0;
-    for (auto& pc : pieces) need += pc.d == d;
-    if (!need) continue;
-    std::vector<Batch*> free_list;
-    for (auto& b : ctx->slots[d]) if (!b->busy) free_list.push_back(b.get());
-    const size_t cap_batches = (size_t)ctx->limits.gofs_in_flight * need;
-    while (free_list.size() < need && ctx->slots[d].size() < cap_batches) {
-      std::unique_ptr<Batch> b(new Batch());
-      if (b->init(ctx->devices[d], ctx->two_pass, err)) return ctx->fail();
-      free_list.push_back(b.get());
-      ctx->slots[d].push_back(std::move(b));
-    }
-    if (free_list.size() < need) {
+  // every piece needs a free batch (GOF slot) of its device
+  for (auto& pc : pieces) {
+    for (auto& b : ctx->slots[pc.d])
+      if (!b->busy) { pc.b = b.get(); break; }
+    if (!pc.b) {
       err.st = TMC2_ERR_STATE;
       err.msg = "all GOF slots in flight: drain frames with tmc2gpu_next_frame / release_frame first";
       return ctx->fail();
     }
-    size_t k = 0;
-    for (auto& pc : pieces) if (pc.d == d) pc.b = free_list[k++];
   }
   // A failure part-way through leaves no trace: pieces already enqueued are drained and freed, and none of the GOF's frames
   // stays in the hand-out queue (a GOF is delivered whole or not at all).
@@ -1410,7 +1390,7 @@ tmc2_status tmc2gpu_submit_gof(tmc2gpu_ctx* ctx, const tmc2_gof* gof) {
     ctx->next_global = global_mark;
   };
   ++ctx->submit_epoch;
-  // The pieces (one per device, or per chunk) are independent batches: digest of the patch lists, staging, H2D and launch
+  // The pieces (one per device) are independent batches: digest of the patch lists, staging, H2D and launch
   // enqueue of every piece run on their own host thread when there are several, so that one submitting thread keeps N devices
   // busy (src/lib.rs has exactly one worker thread above this call).
   std::vector<Err> perr(pieces.size());
@@ -1421,7 +1401,7 @@ tmc2_status tmc2gpu_submit_gof(tmc2gpu_ctx* ctx, const tmc2_gof* gof) {
     TraceClock pt;
     if (b->prepare(gof, pc.lo, pc.hi - pc.lo, 0, e)) return;
     const double t_prep = pt.lap();
-    if (b->upload(gof, pc.lo, dev_ranges, e, pieces.size() == 1)) return;
+    if (b->upload(dev_ranges, e, pieces.size() == 1)) return;
     const double t_up = pt.lap();
     if (b->launch(b->stream, e)) return;
     if (b->enqueue_counts(b->stream, e)) return;          // counts travel right behind the kernels
@@ -1498,45 +1478,35 @@ tmc2_status tmc2gpu_next_frame(tmc2gpu_ctx* ctx, tmc2_frame_out* out) {
   }
   if (b->failed_early.st != TMC2_OK) { err = b->failed_early; b->failed_early = Err(); drop_gof(); return ctx->fail(); }
   const double t_counts = tc.lap();
-  if (ctx->device_output) {
-    // device-resident hand-off: the counts copy was enqueued behind the last kernel of the GOF, so every frame is complete
-    ctx->pending.pop_front();
-    memset(out, 0, sizeof *out);
-    out->frame_index = pf.global_index;
-    out->point_count = b->counts[pf.local];
-    out->positions = reinterpret_cast<const uint16_t*>(b->d_pos.as<uint8_t>() + (size_t)pf.local * b->cap * 6);
-    out->with_colors = b->params.attribute_count ? 1 : 0;
-    out->colors = out->with_colors ? b->d_rgb.as<uint8_t>() + (size_t)pf.local * b->cap * 3 : nullptr;
-    out->memory_space = 1;
-    out->device = (uint8_t)b->device;
-    out->smoothed_positions = b->moved[pf.local];
-    out->smoothed_colors = b->recoloured[pf.local];
-    out->_handle = b;
-    return TMC2_OK;
-  }
-  if (!b->outputs_enqueued && b->enqueue_outputs(err)) { drop_gof(); return ctx->fail(); }
-  const double t_enq = tc.lap();
-  if (cudaSetDevice(b->device) != cudaSuccess || cudaEventSynchronize(b->ev_frame[pf.local]) != cudaSuccess) {
-    err.st = TMC2_ERR_CUDA; err.msg = std::string("waiting for frame: ") + cudaGetErrorString(cudaGetLastError());
-    drop_gof();
-    return ctx->fail();
-  }
-  if (trace_on()) {
-    const double t_wait = tc.lap();
-    b->trace_wait_ms += t_counts + t_enq + t_wait;
-    if (first || pf.local + 1 == b->F)
-      fprintf(stderr, "[tmc2gpu] next_frame local %u: wait-counts %.3f enqueue-d2h %.3f wait-frame %.3f ms | GOF: inside next_frame "
-              "%.3f ms, since submit %.3f ms\n", pf.local, t_counts, t_enq, t_wait, b->trace_wait_ms,
-              std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - b->t_submit).count());
+  // device-resident hand-off: the counts copy was enqueued behind the last kernel of the GOF, so every frame is complete
+  const bool dev = ctx->device_output;
+  if (!dev) {
+    if (!b->outputs_enqueued && b->enqueue_outputs(err)) { drop_gof(); return ctx->fail(); }
+    const double t_enq = tc.lap();
+    if (cudaSetDevice(b->device) != cudaSuccess || cudaEventSynchronize(b->ev_frame[pf.local]) != cudaSuccess) {
+      err.st = TMC2_ERR_CUDA; err.msg = std::string("waiting for frame: ") + cudaGetErrorString(cudaGetLastError());
+      drop_gof();
+      return ctx->fail();
+    }
+    if (trace_on()) {
+      const double t_wait = tc.lap();
+      b->trace_wait_ms += t_counts + t_enq + t_wait;
+      if (first || pf.local + 1 == b->F)
+        fprintf(stderr, "[tmc2gpu] next_frame local %u: wait-counts %.3f enqueue-d2h %.3f wait-frame %.3f ms | GOF: inside next_frame "
+                "%.3f ms, since submit %.3f ms\n", pf.local, t_counts, t_enq, t_wait, b->trace_wait_ms,
+                std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - b->t_submit).count());
+    }
   }
   ctx->pending.pop_front();
   memset(out, 0, sizeof *out);
   out->frame_index = pf.global_index;
   out->point_count = b->counts[pf.local];
-  out->positions = reinterpret_cast<const uint16_t*>(b->h_out.as<uint8_t>() + b->out_pos_off[pf.local]);
+  out->positions = reinterpret_cast<const uint16_t*>(dev ? b->d_pos.as<uint8_t>() + (size_t)pf.local * b->cap * 6
+                                                         : b->h_out.as<uint8_t>() + b->out_pos_off[pf.local]);
   out->with_colors = b->params.attribute_count ? 1 : 0;
-  out->colors = out->with_colors ? b->h_out.as<uint8_t>() + b->out_rgb_off[pf.local] : nullptr;
-  out->memory_space = 0;
+  if (out->with_colors)
+    out->colors = dev ? b->d_rgb.as<uint8_t>() + (size_t)pf.local * b->cap * 3 : b->h_out.as<uint8_t>() + b->out_rgb_off[pf.local];
+  out->memory_space = dev ? 1 : 0;
   out->device = (uint8_t)b->device;
   out->smoothed_positions = b->moved[pf.local];
   out->smoothed_colors = b->recoloured[pf.local];
@@ -1655,7 +1625,7 @@ tmc2_status tmc2gpu_upload_gof(tmc2gpu_ctx* ctx, const tmc2_gof* gof, tmc2_resid
   std::unique_ptr<tmc2_resident> r(new tmc2_resident());
   r->batch.reset(new Batch());
   Batch* b = r->batch.get();
-  if (b->init(ctx->devices[0], ctx->two_pass, err) || b->prepare(gof, 0, gof->frame_count, 0, err) || b->upload(gof, 0, dev_ranges, err))
+  if (b->init(ctx->devices[0], err) || b->prepare(gof, 0, gof->frame_count, 0, err) || b->upload(dev_ranges, err))
     return ctx->fail();
   if (cudaStreamSynchronize(b->stream) != cudaSuccess) { err.st = TMC2_ERR_CUDA; err.msg = "upload sync"; return ctx->fail(); }
   b->h_in.release();   // planes now live in HBM; the staging area is not needed again
@@ -1676,9 +1646,9 @@ tmc2_status tmc2gpu_reconstruct_resident_ex(tmc2gpu_ctx* ctx, tmc2_resident* r, 
   // Relaunches of a resident GOF are the same launch sequence every time: without smoothing (no auxiliary stream, nothing
   // that outlives the launch) it is captured once into a CUDA graph and replayed with one API call -- for a small GOF
   // (BASELINE config 1: one frame, 8 launches + 3 memsets of a few microseconds each) the CPU launch cost is what bounds the
-  // rate.  The first launch and every TMC2_GRAPH=0 launch take the ordinary path, which also records the stage-timing events.
-  static const bool graphs = [] { const char* e = getenv("TMC2_GRAPH"); return !e || atoi(e) != 0; }();
-  const bool eligible = graphs && !(flags & TMC2_LAUNCH_TIMED) && !(b->smoothing_geo || b->smoothing_col) && b->want == 0;
+  // rate.  The first launch and every TMC2_LAUNCH_TIMED launch take the ordinary path, which also records the stage-timing
+  // events.
+  const bool eligible = !(flags & TMC2_LAUNCH_TIMED) && !(b->smoothing_geo || b->smoothing_col) && b->want == 0;
   if (eligible && b->graph_exec) {
     auto replay = [&]() -> tmc2_status {
       CU(cudaSetDevice(b->device));
@@ -1789,7 +1759,8 @@ tmc2_status tmc2gpu_last_stage_ms(tmc2gpu_ctx* ctx, float* ms5) {
   StageTimes t;
   ctx->err = Err();
   if (ctx->last_batch->stage_times(t, ctx->err)) return ctx->fail();
-  ms5[0] = t.b2p; ms5[1] = t.unpack; ms5[2] = t.geo; ms5[3] = t.count; ms5[4] = t.rgb;
+  // ms5[4] = 0: there is no separate YUV -> RGB pass, the conversion is fused into the emit
+  ms5[0] = t.b2p; ms5[1] = t.unpack; ms5[2] = t.geo; ms5[3] = t.count; ms5[4] = 0;
   return TMC2_OK;
 }
 
@@ -1802,7 +1773,7 @@ static tmc2_status run_single(tmc2gpu_ctx* ctx, const tmc2_gof* gof, uint32_t fr
   std::vector<DevRange> dev_ranges;
   if (validate_frame(gof, frame_index, ctx->devices, dev_ranges, err)) return err.st;
   Batch* b = ctx->stage_batch.get();
-  if (b->prepare(gof, frame_index, 1, want, err) || b->upload(gof, frame_index, dev_ranges, err) || b->launch(b->stream, err))
+  if (b->prepare(gof, frame_index, 1, want, err) || b->upload(dev_ranges, err) || b->launch(b->stream, err))
     return err.st;
   if (b->fetch_counts(b->stream, err)) return err.st;
   ctx->last_batch = b;
