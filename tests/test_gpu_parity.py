@@ -28,25 +28,7 @@ def test_appendix_c_known_answer(gpu_ctx):
     assert b2p.tolist() == [1, 2]
 
 
-CASES = [
-    dict(seed=1, orientations=(0, 1)),
-    dict(seed=2, orientations=(0, 1), absolute_d1=False),
-    dict(seed=3, orientations=(0, 1, 8), extreme=True),
-    dict(seed=4, orientations=tuple(range(9)), spec=True),
-    dict(seed=5, orientations=tuple(range(9)), spec=False, n_patches=6),
-    dict(seed=6, orientations=(0, 1), prec=2),
-    dict(seed=7, orientations=(0, 1), prec=1, W=48, H=32),
-    dict(seed=8, orientations=(0, 1, 3, 5), spec=True, res=8, prec=4, W=40, H=32),
-    dict(seed=9, orientations=(0, 1), attr=False),
-    dict(seed=10, orientations=tuple(range(9)), spec=True, absolute_d1=False, extreme=True),
-    dict(seed=11, orientations=(0, 1), W=208, H=112, n_patches=14),
-    dict(seed=12, orientations=tuple(range(9)), spec=True, W=208, H=112, n_patches=14, extreme=True),
-    dict(seed=13, orientations=(0, 1), prec=3, W=48, H=48),
-    dict(seed=14, orientations=(0, 1, 2, 4, 6), spec=False, res=32, W=128, H=96, prec=4),
-]
-
-
-@pytest.mark.parametrize("case", CASES, ids=lambda c: "-".join(f"{k}{v}" for k, v in c.items() if k != "orientations"))
+@pytest.mark.parametrize("case", util.CASES, ids=util.case_id)
 def test_random_small_atlases_bit_exact(gpu_ctx, case):
     g = util.random_small_gof(**case)
     got, want = both(gpu_ctx, g)
@@ -347,10 +329,7 @@ def test_three_entry_points_agree_at_full_size(gpu_ctx):
     assert np.array_equal(frames[0].positions, frames[2].positions) and np.array_equal(frames[1].colors, frames[3].colors)
 
 
-SMOOTH_CASES = [CASES[i] for i in (0, 2, 3, 4, 5, 6, 7, 9, 11, 12, 13)]
-
-
-@pytest.mark.parametrize("case", SMOOTH_CASES, ids=lambda c: "-".join(f"{k}{v}" for k, v in c.items() if k != "orientations"))
+@pytest.mark.parametrize("case", util.SMOOTH_CASES, ids=util.case_id)
 @pytest.mark.parametrize("grids", [(8, 4), (6, 3)], ids=["g8c4", "g6c3"])
 def test_random_small_atlases_with_smoothing(gpu_ctx, case, grids):
     """Every orientation / precision / resolution / no-attribute case again with boundary detection + both smoothing stages
@@ -372,16 +351,7 @@ def test_random_small_atlases_with_smoothing(gpu_ctx, case, grids):
     assert got["smoothed_positions"] == want["smoothed_positions"] and got["smoothed_colors"] == want["smoothed_colors"]
 
 
-FAST_CASES = [
-    dict(seed=21, orientations=(0, 1), W=208, H=112, n_patches=14),
-    dict(seed=22, orientations=tuple(range(9)), spec=True, W=208, H=112, n_patches=14),
-    dict(seed=23, orientations=(0, 1, 8), extreme=True, W=96, H=64, n_patches=8),
-    dict(seed=24, orientations=(0, 1), prec=2, W=64, H=64),
-    dict(seed=25, orientations=(0, 1), absolute_d1=False, W=96, H=64, n_patches=8),
-]
-
-
-@pytest.mark.parametrize("case", FAST_CASES, ids=lambda c: "-".join(f"{k}{v}" for k, v in c.items() if k != "orientations"))
+@pytest.mark.parametrize("case", util.FAST_CASES, ids=util.case_id)
 @pytest.mark.parametrize("content", ["smooth", "noisy", "asis"])
 @pytest.mark.parametrize("grids", [(8, 4), (4, 2), (2, 8)], ids=["g8c4", "g4c2", "g2c8"])
 def test_streaming_smoothing_fast_grids(gpu_ctx, case, content, grids):

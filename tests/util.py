@@ -81,7 +81,46 @@ def _helper(p, u, v, res, sscale):
     return v + u0, u + v0
 
 
-STREAMS = ("positions", "colors", "colors16bit", "partition", "point_to_pixel", "block_to_patch", "occupancy_map")
+# Generator cases: every orientation of both orientation modes, precisions 1-4, resolutions 8 / 16 / 32, widths that are
+# not a multiple of 64, differential D1, u16 wrap and level of detail 2 (`extreme`), and atlases without attributes.
+# tests/test_emit_instantiations.py checks that they reach every emit instantiation and slot path.
+CASES = [
+    dict(seed=1, orientations=(0, 1)),
+    dict(seed=2, orientations=(0, 1), absolute_d1=False),
+    dict(seed=3, orientations=(0, 1, 8), extreme=True),
+    dict(seed=4, orientations=tuple(range(9)), spec=True),
+    dict(seed=5, orientations=tuple(range(9)), spec=False, n_patches=6),
+    dict(seed=6, orientations=(0, 1), prec=2),
+    dict(seed=7, orientations=(0, 1), prec=1, W=48, H=32),
+    dict(seed=8, orientations=(0, 1, 3, 5), spec=True, res=8, prec=4, W=40, H=32),
+    dict(seed=9, orientations=(0, 1), attr=False),
+    dict(seed=10, orientations=tuple(range(9)), spec=True, absolute_d1=False, extreme=True),
+    dict(seed=11, orientations=(0, 1), W=208, H=112, n_patches=14),
+    dict(seed=12, orientations=tuple(range(9)), spec=True, W=208, H=112, n_patches=14, extreme=True),
+    dict(seed=13, orientations=(0, 1), prec=3, W=48, H=48),
+    dict(seed=14, orientations=(0, 1, 2, 4, 6), spec=False, res=32, W=128, H=96, prec=4),
+    # level of detail 2 on the per-pixel slot path (reference-mode rotations are not block-aligned)
+    dict(seed=15, orientations=tuple(range(2, 8)), extreme=True, W=96, H=64, n_patches=8),
+    # no attributes on the occupancy-mask and per-pixel slot paths
+    dict(seed=16, orientations=(0, 1, 2, 5), prec=2, attr=False),
+]
+
+SMOOTH_CASES = [CASES[i] for i in (0, 2, 3, 4, 5, 6, 7, 9, 11, 12, 13)]
+
+FAST_CASES = [
+    dict(seed=21, orientations=(0, 1), W=208, H=112, n_patches=14),
+    dict(seed=22, orientations=tuple(range(9)), spec=True, W=208, H=112, n_patches=14),
+    dict(seed=23, orientations=(0, 1, 8), extreme=True, W=96, H=64, n_patches=8),
+    dict(seed=24, orientations=(0, 1), prec=2, W=64, H=64),
+    dict(seed=25, orientations=(0, 1), absolute_d1=False, W=96, H=64, n_patches=8),
+]
+
+
+def case_id(case):
+    return "-".join(f"{k}{v}" for k, v in case.items() if k != "orientations")
+
+
+STREAMS = ("positions","colors", "colors16bit", "partition", "point_to_pixel", "block_to_patch", "occupancy_map")
 
 
 def assert_same(gpu, orc, keys=STREAMS, what=""):

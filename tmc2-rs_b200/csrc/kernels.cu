@@ -161,9 +161,10 @@ __device__ __forceinline__ ChromaTerm chroma_term(uint32_t U, uint32_t V) {
 }
 // The same three integers for 10-bit chroma from 32-bit arithmetic: 255*k = Cint + Cfrac, Cfrac rounded to 21 fractional bits
 // (error <= 2^-22 per unit of d, so <= 2^-13 over |d| <= 512; the green channel adds two such terms).  The result is exact
-// unless the fraction lands within that error (plus a margin) of 0 or 1 -- about 5 chroma pairs in 10 000, and always for a
+// unless the fraction lands within that error (plus a margin) of 0 or 1 -- 4 603 of the 2^20 chroma pairs, and always for a
 // neutral component (d == 0) -- or the sample is not a 10-bit value; then `flagged` is set and the caller takes chroma_term().
-// Verified exhaustively over all 2^20 (U, V) pairs against exact rational arithmetic (DESIGN.md).
+// Verified exhaustively over all 2^20 (U, V) pairs against exact rational arithmetic in tests/test_fused_colour.py, which
+// also runs every pair through the emit on the luma values where the result turns on these terms.
 __device__ __forceinline__ ChromaTerm chroma_term_fast(uint32_t U, uint32_t V) {
   const uint32_t du = U - 512u, dv = V - 512u;                              // two's complement
   constexpr uint32_t M = (1u << 21) - 1u;
