@@ -114,7 +114,13 @@ typedef struct tmc2_params {
   uint8_t  geometry_smoothing;             /* 1: grid geometry smoothing (needs boundary detection)        */
   uint8_t  color_smoothing;                /* 1: grid colour smoothing on the 16-bit YUV colours           */
   uint8_t  attribute_bitdepth;             /* nominal bit depth of attribute samples (10); scales the      */
-                                           /* colour-smoothing thresholds, which are in 8-bit units        */
+                                           /* colour-smoothing thresholds, which are in 8-bit units, by    */
+                                           /* 2^(bitdepth-8) (1 at 8 and below).  Samples are u16, so with */
+                                           /* colour smoothing on attributes it must be <= 16, else        */
+                                           /* TMC2_ERR_INVALID_ARG.  Colour smoothing also refuses a frame */
+                                           /* whose colour cell holds more than 65 536 type-2 points       */
+                                           /* (TMC2_ERR_UNSUPPORTED): the packed U / V sums are exact up   */
+                                           /* to that count only.                                          */
   uint8_t  _reserved0;
   uint16_t grid_size;                      /* GeometrySmoothingParams._grid_size (SEI grid_size_minus_2+2) */
   uint16_t threshold_smoothing;            /* GeometrySmoothingParams._threshold_smoothing                 */

@@ -165,6 +165,9 @@ static int check_gof(const tmc2_gof* g, uint32_t frame_index) {
   if (P->enable_size_quantization || P->multiple_streams || P->pbf_enabled || P->enhanced_occupancy_map ||
       P->point_local_reconstruction || P->single_map_pixel_interleaving || P->use_additional_points_patch)
     return TMC2_ERR_UNSUPPORTED; /* unimplemented!() codec.rs:285,303,314,399,402,454,494 */
+  /* own spec: colour thresholds scale by 2^(bitdepth-8); samples are u16, so a deeper bit depth means nothing.  Checked
+   * here rather than in color_smoothing so that frames without points are refused too. */
+  if (P->color_smoothing && P->attribute_count && P->attribute_bitdepth > 16) return TMC2_ERR_INVALID_ARG;
   return TMC2_OK;
 }
 

@@ -51,21 +51,22 @@ def _pow2(x):
     return x > 0 and x & (x - 1) == 0
 
 
+def grid_fast(params, g, hashed):
+    """GridDesc.fast of a grid of edge g (tmc2gpu.cu make_args): 0 generic grid, 1 packed 8-bit cell keys, 2 wider."""
+    w = -(-(1 << params.geometry_bitdepth_3d) // g)
+    if hashed or not (_pow2(g) and _pow2(w) and w <= 1024 and g * w <= 65536):
+        return 0
+    return 1 if w <= 256 else 2
+
+
 def emit_instantiation(params, hashed):
     """launch_emit for a launch without debug streams (tmc2gpu.cu fills the GridDesc `fast` field that it reads)."""
     geo = bool(params.geometry_smoothing)
     col = bool(params.color_smoothing) and params.attribute_count != 0
     if not (geo or col):
         return "plain"
-    maxs = 1 << params.geometry_bitdepth_3d
-
-    def grid_fast(g):                      # 0: generic grid, 1: packed 8-bit cell keys, 2: wider
-        w = -(-maxs // g)
-        if hashed or not (_pow2(g) and _pow2(w) and w <= 1024 and g * w <= 65536):
-            return 0
-        return 1 if w <= 256 else 2
-    fast = (not geo or (grid_fast(params.grid_size) == 1 and params.grid_size <= 8)) and \
-           (not col or grid_fast(params.cgrid_size) != 0)
+    fast = (not geo or (grid_fast(params, params.grid_size, hashed) == 1 and params.grid_size <= 8)) and \
+           (not col or grid_fast(params, params.cgrid_size, hashed) != 0)
     return "fast" if fast else "generic"
 
 

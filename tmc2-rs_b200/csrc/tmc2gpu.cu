@@ -287,6 +287,10 @@ static tmc2_status validate_params(const tmc2_gof* g, Err& err) {
   // Image::get asserts (decoder.rs:974): the upsample touches every pixel of the tile
   if ((g->width - 1) / P.occupancy_precision >= g->occ_width || (g->height - 1) / P.occupancy_precision >= g->occ_height)
     FAIL(TMC2_ERR_INVALID_ARG, "occupancy video smaller than frame / precision (decoder.rs:974 assert)");
+  // samples are u16; the colour thresholds are scaled by 2^(bd-8) in 32 bits (make_args).  Checked before the grid limits,
+  // like the oracle's check_gof, so that both report the same status
+  if (P.color_smoothing && P.attribute_count && P.attribute_bitdepth > 16)
+    FAIL(TMC2_ERR_INVALID_ARG, "attribute_bitdepth %u > 16", (unsigned)P.attribute_bitdepth);
   if (P.geometry_smoothing || P.color_smoothing) {
     if (P.geometry_bitdepth_3d == 0 || P.geometry_bitdepth_3d > 16) FAIL(TMC2_ERR_INVALID_ARG, "geometry_bitdepth_3d");
     const uint32_t maxs = 1u << P.geometry_bitdepth_3d;
@@ -1159,7 +1163,8 @@ struct Batch {
       // a slot that bailed out may have claimed cells without marking them touched: the clear pass would miss them, so the
       // next launch of this batch starts from freshly zeroed tables
       geotab_slots = coltab_slots = 0; geotab_frames = coltab_frames = 0;
-      FAIL((tmc2_status)dev_err, "device-side failure flag %d (7 = output capacity, 11 = watchdog / table)", dev_err);
+      FAIL((tmc2_status)dev_err, "device-side failure flag %d (6 = colour cell with more than 65536 type-2 points, 7 = output capacity, "
+                                       "11 = watchdog / table)", dev_err);
     }
     counts.assign(F, 0); moved.assign(F, 0); recoloured.assign(F, 0);
     if (F) {
