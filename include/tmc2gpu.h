@@ -52,7 +52,9 @@ typedef enum tmc2_status {
                                      /*            decoder.rs:271; attribute video < 2 frames codec.rs:589 */
   TMC2_ERR_MAP_COUNT           = 5,  /* reference: map_count != 2 panics at codec.rs:415/:432             */
   TMC2_ERR_UNSUPPORTED         = 6,  /* reference: unimplemented!() branch (pbf, eom, plr, raw, ...)      */
-  TMC2_ERR_CAPACITY            = 7,  /* GOF larger than the limits given to tmc2gpu_create                */
+  TMC2_ERR_CAPACITY            = 7,  /* GOF larger than the limits given to tmc2gpu_create, or than the   */
+                                     /* library's own: width / height >= 32768, occupancy resolution > 64, */
+                                     /* more than 65535 patches in a frame                                */
   TMC2_ERR_STATE               = 8,  /* call order violated (e.g. release of a frame not handed out)      */
   TMC2_ERR_NO_DEVICE           = 9,  /* no CUDA device / bad device id.  There is NO CPU fallback.        */
   TMC2_ERR_CUDA                = 10, /* a CUDA call or kernel failed; see tmc2gpu_last_error              */
@@ -71,7 +73,8 @@ typedef enum tmc2_patch_orientation { /* src/decoder.rs:694-707 */
 
 typedef struct tmc2_patch {
   uint32_t u0, v0;            /* uv0: location in the packed image, in occupancy blocks (pdu.pos_2d)      */
-  uint32_t size_u0, size_v0;  /* size_uv0: size in occupancy blocks (size_2d_minus1 + 1)                  */
+  uint32_t size_u0, size_v0;  /* size_uv0: size in occupancy blocks (size_2d_minus1 + 1); at most 4096     */
+                              /* each, larger is TMC2_ERR_PATCH_OUT_OF_CANVAS                             */
   uint32_t u1, v1;            /* uv1: tangential / bitangential shift (pdu.pos_3d_offset)                 */
   uint32_t d1;                /* depth shift, already mode-adjusted (decoder.rs:468-473)                  */
   uint16_t lod_x, lod_y;      /* level_of_detail; the reference always has (1,1) (decoder.rs:432-436)     */
@@ -95,7 +98,7 @@ typedef enum tmc2_orientation_mode { TMC2_ORIENTATION_REFERENCE = 0, TMC2_ORIENT
  * surface (GeometrySmoothingParams :188-193, ColorSmoothingParams :180-186).
  * ---------------------------------------------------------------------------------------------- */
 typedef struct tmc2_params {
-  uint32_t occupancy_resolution;   /* 1 << log2_patch_packing_block_size (decoder.rs:252,602)              */
+  uint32_t occupancy_resolution;   /* 1 << log2_patch_packing_block_size (decoder.rs:252,602); 1 .. 64     */
   uint32_t occupancy_precision;    /* vps.frame_width / occ.width() (decoder.rs:194)                       */
   uint8_t  map_count_minus1;       /* must be 1 (two maps) -> else TMC2_ERR_MAP_COUNT                      */
   uint8_t  absolute_d1;            /* decoder.rs:605                                                       */
@@ -144,7 +147,7 @@ typedef struct tmc2_frame {
   const uint16_t*   attr_u[2];    /* channel 1, (width/2) x (height/2), 4:2:0                              */
   const uint16_t*   attr_v[2];    /* channel 2                                                             */
   const tmc2_patch* patches;      /* tile.patches, ascending patch index                                   */
-  uint32_t          patch_count;
+  uint32_t          patch_count;  /* at most 65535 (more: TMC2_ERR_CAPACITY)                               */
   uint32_t          occ_stride;   /* >= occ_width                                                          */
   uint32_t          geo_stride;   /* >= width                                                              */
   uint32_t          attr_stride_y;/* >= width                                                              */
@@ -153,8 +156,9 @@ typedef struct tmc2_frame {
 } tmc2_frame;
 
 typedef struct tmc2_gof {
-  uint32_t          width, height;         /* tile.width / tile.height == atlas frame size                 */
-  uint32_t          occ_width, occ_height; /* size of the occupancy video                                  */
+  uint32_t          width, height;         /* tile.width / tile.height == atlas frame size, each < 32768   */
+  uint32_t          occ_width, occ_height; /* size of the occupancy video: at least ceil(width / precision)*/
+                                           /* x ceil(height / precision); samples beyond are not image      */
   uint32_t          frame_count;           /* frames to reconstruct (decoder.rs:188)                       */
   uint32_t          geo_video_frames;      /* atlas.geo_frames[0].frame_count(); must be >= 2*frame_count   */
   uint32_t          attr_video_frames;     /* atlas.attr_frames[0].frame_count()                           */
@@ -203,7 +207,7 @@ typedef struct tmc2_frame_out {
 typedef struct tmc2_limits {
   uint32_t max_width, max_height;  /* largest atlas frame the context must accept                          */
   uint32_t max_frames;             /* largest GOF (frames) accepted by one submit                          */
-  uint32_t max_patches_per_frame;  /* 0 -> default 4096                                                    */
+  uint32_t max_patches_per_frame;  /* accepted for compatibility and not used: a frame may hold 65535      */
   uint32_t gofs_in_flight;         /* submit/next_frame pipelining depth, 0 -> default 2                   */
   uint32_t flags;                  /* TMC2_CTX_* bits                                                      */
 } tmc2_limits;

@@ -154,18 +154,6 @@ def test_smoothing_spec_invariants():
     assert rec.sum() == a["smoothed_colors"]
     assert (a["boundary_type"][rec] == 1).all()
     # boundary types against a direct numpy evaluation of the spec
-    occ = a["occupancy_map"] != 0
-    H, W = occ.shape
-    pad = np.pad(occ, 1, constant_values=False)
-    four = pad[1:-1, :-2] & pad[1:-1, 2:] & pad[:-2, 1:-1] & pad[2:, 1:-1]
-    border = np.zeros_like(occ)
-    border[0, :] = border[-1, :] = border[:, 0] = border[:, -1] = True
-    t1 = occ & (border | ~four)
-    pad2 = np.pad(occ, 2, constant_values=True)
-    all5 = np.ones_like(occ)
-    for dy in range(5):
-        for dx in range(5):
-            all5 &= pad2[dy:dy + H, dx:dx + W]
-    expect = np.where(t1, 1, np.where(occ & ~all5, 2, 0))
+    expect = util.boundary_spec(a["occupancy_map"])
     px = a["point_to_pixel"]
     assert np.array_equal(a["boundary_type"], expect[px[:, 1], px[:, 0]])

@@ -6,8 +6,12 @@ from tmc2rs_b200 import abi, synth
 
 
 def random_small_gof(seed, W=64, H=48, frames=1, orientations=(0, 1), spec=False, absolute_d1=True, res=16, prec=4,
-                     n_patches=5, attr=True, depth_max=250, extreme=False):
+                     n_patches=5, attr=True, depth_max=250, extreme=False, slack=(0, 0), slack_fill=0):
     """A small atlas with random (possibly overlapping) patches of the given orientations.
+
+    The occupancy video is ceil(W / prec) x ceil(H / prec) samples, plus `slack` = (columns, rows) more filled with
+    `slack_fill`: a decoder's occupancy video may be larger than the atlas needs, and those samples are not image.  W and
+    H may be odd (then without attributes: 4:2:0 planes need even sizes).
 
     Patch placement keeps every pixel of every patch inside the canvas under the chosen orientation mode (in REFERENCE
     mode the rotated orientations use the reference's un-scaled sizes, so their pixel footprint differs from the block
@@ -47,7 +51,10 @@ def random_small_gof(seed, W=64, H=48, frames=1, orientations=(0, 1), spec=False
             lod = (1, 1) if not extreme else (int(rng.randint(1, 3)), int(rng.randint(1, 3)))
             plist.append((u0, v0, su, sv, u1, v1, d1, lod[0], lod[1], n, t, b, mode, o, 0, (0, 0)))
         patch_lists.append(np.array(plist, dtype=abi.PATCH_DTYPE))
-    occ = (rng.rand(frames, H // prec, W // prec) < 0.6).astype(np.uint8) * rng.randint(1, 256, (frames, H // prec, W // prec)).astype(np.uint8)
+    oh, ow = -(-H // prec), -(-W // prec)
+    occ = (rng.rand(frames, oh, ow) < 0.6).astype(np.uint8) * rng.randint(1, 256, (frames, oh, ow)).astype(np.uint8)
+    if slack != (0, 0):
+        occ = np.pad(occ, ((0, 0), (0, slack[1]), (0, slack[0])), constant_values=slack_fill)
     d0 = rng.randint(0, depth_max, (frames, H, W))
     delta = np.where(rng.rand(frames, H, W) < 0.4, 0, rng.randint(1, 5, (frames, H, W)))
     geo = np.empty((frames, 2, H, W), np.uint16)
@@ -134,6 +141,25 @@ def assert_same(gpu, orc, keys=STREAMS, what=""):
             bad = np.argwhere(a.astype(np.int64) != b.astype(np.int64))
             raise AssertionError(f"{what}: {k} differs at {len(bad)} entries, first {bad[0].tolist()}: "
                                  f"gpu {a[tuple(bad[0])]} oracle {b[tuple(bad[0])]}")
+
+
+def boundary_spec(occ):
+    """Boundary class of every pixel of a full-resolution occupancy map (H x W, the image only), straight from the
+    specification (DESIGN.md section 5): 1 = occupied on the image border or with an unoccupied 4-neighbour, 2 = another
+    occupied pixel with an unoccupied pixel in its 5 x 5 window (clipped to the image), 0 = the rest."""
+    occ = occ != 0
+    H, W = occ.shape
+    pad = np.pad(occ, 1, constant_values=False)
+    four = pad[1:-1, :-2] & pad[1:-1, 2:] & pad[:-2, 1:-1] & pad[2:, 1:-1]
+    border = np.zeros_like(occ)
+    border[0, :] = border[-1, :] = border[:, 0] = border[:, -1] = True
+    t1 = occ & (border | ~four)
+    pad2 = np.pad(occ, 2, constant_values=True)
+    all5 = np.ones_like(occ)
+    for dy in range(5):
+        for dx in range(5):
+            all5 &= pad2[dy:dy + H, dx:dx + W]
+    return np.where(t1, 1, np.where(occ & ~all5, 2, 0))
 
 
 def crowd_into_one_region(g):
