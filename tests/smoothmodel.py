@@ -84,8 +84,44 @@ def _stats(points, grid):
     return cells
 
 
-def smooth(params, positions, colors, partition, btype):
+def _merge(cells, prior, g=None):
+    """Add leftover cell statistics (cell_statistics) into `cells`.  A leftover cell lands on the cell with the same
+    coordinates (the key of a hashed table, and the dense index cx + w*(cy + w*cz) when the slot count is the same); its
+    patch set joins the cell's, because its claim word still holds `patch + 1`.  Geometry sums are kept relative to the cell
+    origin (as the tables hold them), so they are re-based on this grid's origin of that cell (`g`)."""
+    for c, (cnt, sums, patches) in prior.items():
+        if g is not None:
+            sums = [s + cnt * c[a] * g for a, s in enumerate(sums)]
+        e = cells.setdefault(c, {"count": 0, "sums": [0] * len(sums), "patches": set()})
+        e["count"] += cnt
+        e["sums"] = [a + b for a, b in zip(e["sums"], sums)]
+        e["patches"] |= set(patches)
+
+
+def cell_statistics(params, positions, colors, partition, btype):
+    """What one frame leaves in the cell tables when nothing clears them: {"geo": {cell: (count, sums relative to the cell
+    origin, patches)}, "col": {cell: (count, [sum Y, sum U, sum V, sum Y^2], patches)}}.  The patch identity is the index of
+    the patch within its frame (what the claim word holds, minus one)."""
+    pos = [tuple(int(c) for c in p) for p in positions]
+    part = [int(x) for x in partition]
+    bt = [int(x) for x in btype]
+    out = {"geo": {}, "col": {}}
+    if params.geometry_smoothing:
+        G = Grid(params.grid_size, params.geometry_bitdepth_3d)
+        for c, e in _stats([(pos[k], part[k], pos[k]) for k in range(len(pos))], G).items():
+            out["geo"][c] = (e["count"], [s - e["count"] * c[a] * G.g for a, s in enumerate(e["sums"])], e["patches"])
+    if params.color_smoothing and colors is not None and params.attribute_count:
+        G = Grid(params.cgrid_size, params.geometry_bitdepth_3d)
+        col = [tuple(int(c) for c in x) for x in colors]
+        pts = [(pos[k], part[k], (col[k][0], col[k][1], col[k][2], col[k][0] ** 2)) for k in range(len(pos)) if bt[k] == 2]
+        out["col"] = {c: (e["count"], e["sums"], e["patches"]) for c, e in _stats(pts, G).items()}
+    return out
+
+
+def smooth(params, positions, colors, partition, btype, prior=None):
     """positions / colors: sequences of 3 ints per point (colors may be None), partition / btype: one int per point.
+    prior: leftover cell statistics of an earlier frame (cell_statistics), merged into the cells before the filters run --
+    the tables of a launch whose cells were not cleared.
 
     Returns dict(positions, colors, moved, recoloured, geo, col, type2_per_cell) where geo / col map the point index of
     every type-1 point that reached a comparison to its quantities."""
@@ -101,6 +137,8 @@ def smooth(params, positions, colors, partition, btype):
     if params.geometry_smoothing:
         G = Grid(params.grid_size, params.geometry_bitdepth_3d)
         cells = _stats([(pos[k], part[k], pos[k]) for k in range(n)], G)
+        if prior:
+            _merge(cells, prior.get("geo", {}), G.g)
         thr = params.threshold_smoothing
         for k in range(n):
             p = pos[k]
@@ -137,6 +175,8 @@ def smooth(params, positions, colors, partition, btype):
         t_var = params.threshold_color_variation * sc
         pts = [(pos[k], part[k], (col[k][0], col[k][1], col[k][2], col[k][0] ** 2)) for k in range(n) if bt[k] == 2]
         cells = _stats(pts, G)
+        if prior:
+            _merge(cells, prior.get("col", {}))
         for c, e in cells.items():
             type2[c] = e["count"]
         for k in range(n):
@@ -175,10 +215,19 @@ def smooth(params, positions, colors, partition, btype):
                 type2_per_cell=type2)
 
 
-def smooth_oracle_frame(params, frame):
-    """smooth() on the pre-smoothing streams of an oracle frame (oracle.reconstruct_frame)."""
+def _presmooth(frame):
     colors = frame["colors16bit_presmooth"] if frame["with_colors"] and len(frame["colors16bit_presmooth"]) else None
     if colors is None and frame["with_colors"]:
         colors = frame["colors16bit"]
-    return smooth(params, frame["positions_presmooth"].tolist(), None if colors is None else colors.tolist(),
-                  frame["partition"].tolist(), frame["boundary_type"].tolist())
+    return (frame["positions_presmooth"].tolist(), None if colors is None else colors.tolist(), frame["partition"].tolist(),
+            frame["boundary_type"].tolist())
+
+
+def smooth_oracle_frame(params, frame, prior=None):
+    """smooth() on the pre-smoothing streams of an oracle frame (oracle.reconstruct_frame)."""
+    return smooth(params, *_presmooth(frame), prior=prior)
+
+
+def oracle_frame_statistics(params, frame):
+    """cell_statistics() of an oracle frame, under `params` (the grids of the launch that left them)."""
+    return cell_statistics(params, *_presmooth(frame))

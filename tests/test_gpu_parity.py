@@ -495,11 +495,11 @@ def test_failed_gof_is_dropped_whole_and_slot_is_freed():
             ctx.next_frame()
         assert ctx.next_frame() is None                                    # nothing of the failed GOF is left
         os.environ.pop("TMC2_TEST_BLIST_CAP")
-        g.params.geometry_smoothing = False
-        g.params.color_smoothing = False
-        frames = ctx.decode_gof(abi.GofView(g))                            # the single slot is usable again
-        want = oracle.reconstruct_frame(abi.GofView(g), 1)
-        assert np.array_equal(frames[1].positions, want["positions"])
+        frames = ctx.decode_gof(view)          # the single slot is usable again, and smoothing on it is right
+        for f, fr in enumerate(frames):
+            want = oracle.reconstruct_frame(view, f)
+            assert np.array_equal(fr.positions, want["positions"]) and np.array_equal(fr.colors, want["colors"]), f
+            assert (fr.smoothed_positions, fr.smoothed_colors) == (want["smoothed_positions"], want["smoothed_colors"]), f
     finally:
         os.environ.pop("TMC2_TEST_BLIST_CAP", None)
         ctx.close()
